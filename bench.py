@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the P25 baseband hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1], unchanged since round 1 so that rounds stay comparable): 1,024 independent
@@ -30,6 +30,13 @@ and phase-continuous, so consecutive steps are a continuous transmission and eve
 The timed steps are checked: events of a deterministic sample of streams (first, last, CTA-boundary straddlers) over
 the warm-up and every timed step must equal the oracle's, not just carry valid CRCs.
 
+--dump-outputs DIR writes what the last timed step of the headline workload handed back (rank 0), so that two builds can
+be compared output for output on the same seeded input:
+  events_fields.npy   float64 [N][4]   stream, kind, sample, len of every event of that step, ordered by (stream, sample)
+  events_payload.npy  float32 [N][60]  their payload bytes
+  baseband.npy        float32 [k][n]   the step's 48 kHz baseband of the dumped streams (read back from the device)
+  streams.npy         float64 [k]      the dumped streams: all of them, or a fixed seeded sample that keeps DIR under 64 MB
+
 Multi-GPU: streams shard by rank with no collective on the data path (SURVEY.md section 8e).  torch.distributed (NCCL)
 is used only for the barrier and the MAX of the per-rank device times.
 """
@@ -44,6 +51,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is cached beside the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "spec")):
     if p not in sys.path:
@@ -420,7 +428,29 @@ class OracleSample:
         return {"streams": len(self.streams), "oracle_events": len(ref), "gpu_events": len(got), "differing": len(a ^ b)}
 
 
-def measure(wl: Workload, rank: int, local: int, K: int, W: int, barrier, gate_on: bool, verify: bool, sustained_s: float, Ke: int):
+DUMP_LIMIT = 64_000_000               # bytes --dump-outputs may write
+DUMP_EVENT_BYTES = 4 * 8 + 60 * 4     # one event row of events_fields + events_payload
+
+
+def last_step_outputs(ctx, wl: Workload, drained, steps_done: int) -> dict:
+    """Events and baseband of the last step (see --dump-outputs).  `drained` holds the packed polls that collected it."""
+    import p25rx_b200 as p25
+    n_out, S = wl.n // wl.decim, wl.streams
+    k = min(S, (DUMP_LIMIT - 4096) // (4 * n_out + 2 * wl.slot_events * DUMP_EVENT_BYTES))   # room for twice the usual events
+    streams = np.arange(S) if k == S else np.sort(np.random.default_rng(0).choice(S, k, replace=False))
+    ev = np.concatenate([ctx.unpack(w, ne) for w, ne in drained] + [np.zeros(0, dtype=p25.EVENT_DTYPE)])
+    ev = ev[(ev["sample"] >= (steps_done - 1) * n_out) & np.isin(ev["stream"], streams)]
+    ev = ev[np.lexsort((ev["sample"], ev["stream"]))]
+    out = {"events_fields": np.stack([ev["stream"], ev["kind"], ev["sample"], ev["len"]], axis=1).astype(np.float64),
+           "events_payload": ev["payload"].astype(np.float32),
+           "baseband": np.stack([ctx.read_baseband(int(s), n_out) for s in streams]),
+           "streams": streams.astype(np.float64)}
+    assert sum(a.nbytes + 128 for a in out.values()) <= DUMP_LIMIT, {n: a.shape for n, a in out.items()}
+    return out
+
+
+def measure(wl: Workload, rank: int, local: int, K: int, W: int, barrier, gate_on: bool, verify: bool, sustained_s: float, Ke: int,
+            dump: bool = False):
     """All device legs of one workload on this rank.  Returns a dict of per-rank times / counts (caller reduces)."""
     import torch
     import p25rx_b200 as p25
@@ -487,6 +517,8 @@ def measure(wl: Workload, rank: int, local: int, K: int, W: int, barrier, gate_o
     out["dev_ms"] = t_begin.elapsed_time(t_end)
     out["ddc_ms"], n_timed = ctx.demod_timing(False)     # the library's own event pair right around each kernel launch
     assert n_timed == min(K, 128)
+    if dump:
+        out["dump"] = last_step_outputs(ctx, wl, raw, W + K)
     n_events += burst_events
     # ---------------- sampled-oracle check of the warm-up and every timed step
     if orc is not None:
@@ -697,9 +729,14 @@ def run_b200(args):
     wl = Workload(args.workload, world)
     sampler = ClockSampler(local)
     sampler.start()
-    m = reduce_max(measure(wl, rank, local, K, W, barrier, not args.no_gate, not args.no_verify, args.sustained, args.e2e_steps))
+    m = reduce_max(measure(wl, rank, local, K, W, barrier, not args.no_gate, not args.no_verify, args.sustained, args.e2e_steps,
+                           dump=args.dump_outputs is not None and rank == 0))
     sampler.stop_flag = True
     sampler.join()
+    if "dump" in m:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in m.pop("dump").items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     head = summarise(wl, m, world, K, hbm, hbm_src, fp32, h2d_gbs)
     line = {"metric": METRIC, "value": head["value"], "unit": "Msamples/s", "n_gpus": world, "steps": K, "warmup": W,
             "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": wl.scaling, "vs_baseline": None, "dtype": "f32",
@@ -734,7 +771,7 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)
+    ap.add_argument("--steps", type=int, default=40, help="timed steps of the headline workload (`value`)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
@@ -746,7 +783,13 @@ def main():
                     help="headline workload (default cfg2 = BASELINE configs[1], the configuration the metric is quoted on)")
     ap.add_argument("--extra", default=None, help=f"comma list of further workloads reported under `workloads` (default: {EXTRA_DEFAULT} "
                                                   "when the headline is cfg2; '' for none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the events and baseband of the last timed step of the headline workload to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs dumps the GPU path (--impl b200)")
     if args.extra is None:
         args.extra = EXTRA_DEFAULT if args.workload == "cfg2" and args.impl == "b200" else ""
     if args.impl == "reference":

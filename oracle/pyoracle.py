@@ -6,9 +6,12 @@ product package p25rx_b200 never imports this module.
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -21,14 +24,25 @@ EVENT_DTYPE = np.dtype([("stream", "<u4"), ("kind", "<u4"), ("sample", "<u8"), (
 assert EVENT_DTYPE.itemsize == 80
 
 
+_native_dir: str | None = None
+
+
 def build(native: bool = False) -> str:
-    """(Re)build the oracle if its sources are newer than the library."""
-    name = "libp25oracle_native.so" if native else "libp25oracle.so"
-    path = os.path.join(HERE, name)
+    """(Re)build the oracle if its sources are newer than the library.  The -march=native copy is built once per process
+    into a temporary directory: it fits only the host it was compiled on, and the source tree may be read-only."""
+    global _native_dir
+    if native:
+        if _native_dir is None:
+            d = tempfile.mkdtemp(prefix="p25oracle-")
+            atexit.register(shutil.rmtree, d, ignore_errors=True)
+            subprocess.check_call(["make", "-C", HERE, "native", "NATIVE_LIB=" + os.path.join(d, "libp25oracle_native.so")],
+                                  stdout=subprocess.DEVNULL)
+            _native_dir = d
+        return os.path.join(_native_dir, "libp25oracle_native.so")
+    path = os.path.join(HERE, "libp25oracle.so")
     srcs = [os.path.join(HERE, f) for f in ("p25_oracle.cpp", "p25_oracle.hpp", "p25_tables.h", "Makefile")]
     if not os.path.exists(path) or any(os.path.getmtime(s) > os.path.getmtime(path) for s in srcs):
-        subprocess.check_call(["make", "-C", HERE, "native" if native else "all"],
-                              stdout=subprocess.DEVNULL)
+        subprocess.check_call(["make", "-C", HERE, "all"], stdout=subprocess.DEVNULL)
     return path
 
 

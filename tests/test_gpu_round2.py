@@ -386,7 +386,7 @@ def test_contexts_on_two_devices_in_one_process(p25, oracle):
     its own host thread, fast kernels with opted-in dynamic shared memory on both devices."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     _two_context_case(p25, oracle, [1, 0, 1, 0])
 
 
