@@ -11,27 +11,25 @@
 //
 // The whole chain is non-recursive, so every output is a pure function of a window of the logical
 // input (tail of the previous chunk ++ this chunk); the only carried state is that raw input tail,
-// kept in the stream's own sample format.  Four kernels share the arithmetic:
+// kept in the stream's own sample format.  Five kernels share the arithmetic:
 //
 //   p25_ddc_fm_kernel<FRONT,FMT>      generic: any length and alignment, the first chunk of a stream
 //                                     (implicit zeros in front of it), odd chunks.  A CTA owns one
 //                                     (stream, segment), stages blocks with coalesced loads (u8 through
 //                                     a shared-memory copy of the table), runs the decimating stages
 //                                     input-stationary and the 48 kHz stages on power-of-two rings.
-//   fast::p25_ddc_fm_stream_kernel    cf32, /50 (the bench kernel): TMA bulk copies into a two-stage
-//                                     ring, FFMA2 FIRs, persistent grid with a static + ticket work split.
-//   fast5::p25_ddc5_fm_kernel<FMT>    /5 tile kernel: independent tiles with their own warm-up.
-//   w5::p25_ddc5_warp_kernel<FMT>     /5 warp-autonomous kernel (default for cf32): every warp is
-//                                     its own pipeline, no CTA barriers.
-//   w5i::p25_ddc5_imma_kernel         u8 /5 (default): the warp kernel with the /5 decimator as exact integer
+//   fast::p25_ddc_fm_stream_kernel    /50: cf32 (the bench kernel), and u8 chunks shorter than the tail.
+//                                     TMA bulk copies into a two-stage ring, FFMA2 FIRs, persistent grid
+//                                     with a static + ticket work split.
+//   w5::p25_ddc5_warp_kernel          cf32 /5: warp-autonomous, every warp is its own pipeline, no CTA
+//                                     barriers.
+//   w5i::p25_ddc5_imma_kernel         u8 /5: the warp kernel with the /5 decimator as exact integer
 //                                     products on the tensor pipe (mma.sync u8 x s8 on the raw IQ bytes).
-//   w50i::p25_ddc50_imma_kernel       u8 /50 (default): both decimating stages as one 290-tap integer FIR.
+//   w50i::p25_ddc50_imma_kernel       u8 /50: both decimating stages as one 290-tap integer FIR.
 //
 // Algorithmic traffic: 8 + 4/D bytes per cf32 input sample, 2 + 4/D per u8 sample (DESIGN.md sec. 4); the cf32 /50
 // kernel is HBM-bound (97 %), u8 /50 runs at 78 % of HBM, the /5 kernels are bound by issue slots and the FP32 pipe
 // (62 complex-by-real taps per output; u8: 41 once the decimator is on the tensor pipe).
-#include <stdlib.h>
-
 #include "p25cu_internal.cuh"
 #include "p25_imma_tables.h"
 
@@ -677,90 +675,6 @@ __global__ void __maxnreg__(F<FMT>::MAXREG) p25_ddc_fm_stream_kernel(const DdcPa
   }
 }
 
-}  // namespace fast
-
-
-// =====================================================================================================
-// Fast path for the reference's own chain (/5 from 240 kS/s; u8 or cf32 input; 16-byte aligned rows).
-// At 2.8 bytes per input sample the FP32 pipe, not HBM, is the first limit of this shape (66 complex-by-
-// real taps per 48 kHz output, SURVEY.md section 8d), so the kernel is organised around issue slots:
-//   * tiles of MB outputs are independent: a tile recomputes its own 50-output warm-up (40 channel-filter
-//     taps + discriminator + boxcar) from raw input, so there is no carried on-chip state and every CTA of
-//     the persistent grid simply walks its share of the flattened (stream, tile) space;
-//   * the raw tile (u8 pairs or cf32) is staged by TMA 1-D bulk copies into a two-stage ring;
-//   * decimator: a thread owns 5R consecutive inputs, converts them once (u8: PRMT into the mantissa of
-//     2^23, one packed add) and forms its R outputs' own part plus the part it contributes to its left
-//     neighbour's last four outputs; neighbours exchange by warp shuffle (lane 31 of a warp is a ghost whose
-//     outputs belong to lane 0 of the next warp).  25 FFMA2 per output, no redundant conversion;
-//   * channel filter: 6 outputs per thread from a sliding register window (23 LDS.128 per 246 FFMA2);
-//   * u8 samples stay in byte units, centred on 128: the discriminator is scale-invariant, the remaining
-//     DC of (0.5 / 127.5) is added back as the channel filter's initial accumulator, power is rescaled.
-// =====================================================================================================
-namespace fast5 {
-
-using fast::cfma;
-using fast::mbar_init;
-using fast::mbar_expect_tx;
-using fast::mbar_wait;
-using fast::tma_load_1d;
-
-template <int FMT>
-struct K {
-    static constexpr bool U8 = FMT == P25CU_FMT_U8_IQ;
-    static constexpr int NW = 6, NT = 32 * NW;
-    static constexpr int R = U8 ? 4 : 5;                       // decimator outputs per thread
-    static constexpr int NYD = NW * 31 * R;                    // decimator outputs per tile
-    static constexpr int HC = P25_TAPS_CHAN - 1;               // 40
-    static constexpr int HALO = HC + 1 + (P25_BOXCAR - 1);     // 50 warm-up outputs
-    static constexpr int MB = NYD - HALO;                      // stored outputs per tile
-    static constexpr int XN = 5 * NYD + 5 * R;                 // input samples read per tile (incl. the last ghost lane)
-    static constexpr int AL = U8 ? 8 : 2;                      // samples per 16 bytes
-    static constexpr int ES = U8 ? 2 : 8;                      // bytes per sample
-    static constexpr int XLEN = (XN + 2 * AL - 2) / AL * AL;   // staged samples: XN + alignment skew, whole 16-byte groups
-    static constexpr int XBYTES = (XLEN * ES + 127) / 128 * 128;
-    static constexpr int RC = 6;                               // channel-filter outputs per thread
-    static constexpr int NC = NYD - HC;                        // channel-filter outputs per tile
-    static constexpr int NCT = (NC + RC - 1) / RC;             // threads busy in the channel filter
-    static constexpr int ND = NC - 1;                          // discriminator outputs per tile
-    static_assert(MB % 2 == 0 && (R % 2 == 0 || !U8), "pair stores / word-aligned u8 columns");
-    static_assert(NCT <= NT, "channel filter must fit one pass");
-};
-
-template <int FMT>
-struct __align__(128) Smem {
-    using C = K<FMT>;
-    unsigned char xs[2][C::XBYTES];      // TMA destinations (raw samples)
-    float2 yd[C::NCT * C::RC + C::HC + 2];   // decimator outputs (padded for the last channel-filter thread)
-    float2 c[C::NCT * C::RC + 6];
-    float d[C::ND + 20];
-    unsigned long long full[2];
-};
-
-using fast::add2;
-
-// atan2 for the discriminator: |error| <= 2e-7 rad (degree-7 minimax in t^2 on [0, 1], spec/gen_tables.py
-// style fit; CUDA's atan2f costs ~85 instructions with its special-case branches, this one ~22, branch-free).
-// atan2(0, 0) = 0 like std::atan2 on +0 arguments.
-__device__ __forceinline__ float disc_atan2(float y, float x) {
-    const float ax = fabsf(x), ay = fabsf(y);
-    const float mx = fmaxf(ax, ay), mn = fminf(ax, ay);
-    float rc;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc) : "f"(fmaxf(mx, 1e-30f)));
-    const float t = mn * rc, u = t * t;
-    float q = -0.004295386839658022f;
-    q = fmaf(q, u, 0.022737378254532814f);
-    q = fmaf(q, u, -0.057179518043994904f);
-    q = fmaf(q, u, 0.09735459089279175f);
-    q = fmaf(q, u, -0.13945257663726807f);
-    q = fmaf(q, u, 0.1995391547679901f);
-    q = fmaf(q, u, -0.3333050608634949f);
-    q = fmaf(q, u, 0.9999995231628418f);
-    float r = q * t;
-    r = ay > ax ? 1.57079632679489662f - r : r;
-    r = x < 0.f ? 3.14159265358979324f - r : r;
-    return copysignf(r, y);
-}
-
 __device__ __forceinline__ float2 mul2(float2 a, float2 b) {
     unsigned long long r;
     asm("mul.rn.f32x2 %0, %1, %2;"
@@ -777,7 +691,10 @@ __device__ __forceinline__ float2 fma2s(float2 a, float2 b, float c) {   // a * 
           "l"(*reinterpret_cast<const unsigned long long*>(&cc)));
     return *reinterpret_cast<float2*>(&r);
 }
-// disc_atan2 for two outputs at once: the polynomial and the three multiplies run packed (same arithmetic per half)
+// atan2 for the discriminator, two outputs at once: |error| <= 2e-7 rad (degree-7 minimax in t^2 on [0, 1], spec/gen_tables.py
+// style fit; CUDA's atan2f costs ~85 instructions with its special-case branches, this one ~22, branch-free).
+// atan2(0, 0) = 0 like std::atan2 on +0 arguments.  The polynomial and the three multiplies run packed (same arithmetic
+// per half).
 __device__ __forceinline__ float2 disc_atan2_pair(float2 y, float2 x) {
     const float ax0 = fabsf(x.x), ay0 = fabsf(y.x), ax1 = fabsf(x.y), ay1 = fabsf(y.y);
     const float mx0 = fmaxf(ax0, ay0), mn0 = fminf(ax0, ay0), mx1 = fmaxf(ax1, ay1), mn1 = fminf(ax1, ay1);
@@ -802,210 +719,20 @@ __device__ __forceinline__ float2 disc_atan2_pair(float2 y, float2 x) {
     return make_float2(copysignf(r0, y.x), copysignf(r1, y.y));
 }
 
-// 5R u8 samples starting at half-word ODD of wp[0] -> floats in byte units centred on 128
-template <int R, bool ODD>
-__device__ __forceinline__ void load_u8(const unsigned* __restrict__ wp, float2 (&x)[5 * R]) {
-    fast::load_u8n<5 * R, ODD>(wp, x);
-}
-
-// bulk copies of logical samples [l0 - skew, ...) covering the tile's window into xs[stage]
-template <int FMT>
-__device__ __forceinline__ void issue_tile(Smem<FMT>& sm, int stage, const DdcParams& p, const unsigned char* tail,
-                                           const unsigned char* chunk, int l0) {
-    using C = K<FMT>;
-    const long long ht = p.ht, lend = ht + (long long)p.n;
-    const long long la = (long long)(l0 & ~(C::AL - 1));
-    long long lb = la + C::XLEN;
-    if (lb > lend) lb = lend;
-    const long long t1 = lb < ht ? lb : ht;
-    const unsigned nt = la < t1 ? (unsigned)(t1 - la) : 0u;     // samples served by the tail
-    const long long cb = la > ht ? la : ht;
-    const unsigned nc = cb < lb ? (unsigned)(lb - cb) : 0u;     // samples served by the chunk
-    mbar_expect_tx(&sm.full[stage], (nt + nc) * C::ES);
-    if (nt) tma_load_1d(&sm.xs[stage][0], tail + la * C::ES, nt * C::ES, &sm.full[stage]);
-    if (nc) tma_load_1d(&sm.xs[stage][(cb - la) * C::ES], chunk + (cb - ht) * C::ES, nc * C::ES, &sm.full[stage]);
-}
-
-template <int FMT>
-__global__ void __launch_bounds__(K<FMT>::NT) p25_ddc5_fm_kernel(const DdcParams p, const unsigned tiles_per_stream,
-                                                                   const float dc, const float pw_scale) {
-    using C = K<FMT>;
-    constexpr int R = C::R;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    Smem<FMT>& sm = *reinterpret_cast<Smem<FMT>*>(smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-
-    if (tid == 0) {
-        mbar_init(&sm.full[0], 1);
-        mbar_init(&sm.full[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    // this CTA's share of the flattened (stream, tile) space; (s, it) advance incrementally
-    const unsigned long long total = (unsigned long long)p.n_streams * tiles_per_stream;
-    const unsigned long long b0 = total * blockIdx.x / gridDim.x;
-    const unsigned n_tiles = (unsigned)(total * (blockIdx.x + 1ull) / gridDim.x - b0);
-    const int M0n = (int)p.n_out;
-    const size_t row_bytes = (size_t)p.n * C::ES, tail_bytes = (size_t)p.ht * C::ES;
-    const unsigned char* const iq8 = (const unsigned char*)p.iq;
-    const unsigned char* const tail8 = (const unsigned char*)p.tail_in;
-    // logical index (tail ++ chunk) of the first input of tile `it`: absolute input 5 * (m_lo - HALO) - 20
-    const int l_base = (int)(5 * (long long)p.m0 - (long long)p.a0) - 5 * C::HALO - 20 + (int)p.ht;
-    auto tile_l0 = [&](unsigned it) { return l_base + 5 * C::MB * (int)it; };
-    unsigned s = (unsigned)(b0 / tiles_per_stream), it = (unsigned)(b0 % tiles_per_stream);
-    __syncthreads();
-    if (tid == 0) {
-        unsigned s2 = s, it2 = it;
-        for (unsigned k = 0; k < 2 && k < n_tiles; k++) {
-            issue_tile<FMT>(sm, (int)k, p, tail8 + s2 * tail_bytes, iq8 + s2 * row_bytes, tile_l0(it2));
-            if (++it2 == tiles_per_stream) it2 = 0, s2++;
-        }
-    }
-
-    for (unsigned use = 0; use < n_tiles; use++) {
-        const int stage = use & 1;
-        const int l0 = tile_l0(it);
-        const int skew = l0 & (C::AL - 1);
-        const int m_rel = C::MB * (int)it;                            // first stored output of this tile, relative to m0
-        const int nv = min(M0n - m_rel, C::MB);                       // stored outputs of this tile
-        mbar_wait(&sm.full[stage], (use >> 1) & 1);
-
-        // ---- /5 decimator: column tq owns inputs [5R*tq, 5R*tq + 5R) of the window
-        {
-            const int tq = warp * 31 + lane;
-            float2 x[5 * R];
-            if constexpr (C::U8) {
-                const int s0 = skew + 5 * R * tq;
-                const unsigned* wp = reinterpret_cast<const unsigned*>(sm.xs[stage]) + (s0 >> 1);
-                if (s0 & 1) load_u8<R, true>(wp, x);
-                else load_u8<R, false>(wp, x);
-            } else {
-                const float2* xp = reinterpret_cast<const float2*>(sm.xs[stage]) + skew + 5 * R * tq;
-#pragma unroll
-                for (int i = 0; i < 5 * R; i++) x[i] = xp[i];
-            }
-            float2 own[R], left[R];
-#pragma unroll
-            for (int r = 0; r < R; r++) {
-                own[r] = make_float2(0.f, 0.f);
-                left[r] = make_float2(0.f, 0.f);
-#pragma unroll
-                for (int k = P25_TAPS_DECIM - 1; k >= 0; k--) {      // oldest input first
-                    if ((P25_TAPS_DECIM_ZERO_MASK >> k) & 1) continue;  // taps that are zero to working precision
-                    const int idx = 5 * r + (P25_TAPS_DECIM - 1) - k;
-                    if (idx < 5 * R) own[r] = cfma(c_taps_decim[k], x[idx], own[r]);
-                    else left[r] = cfma(c_taps_decim[k], x[idx - 5 * R], left[r]);
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < R; r++) {
-                if (5 * r + (P25_TAPS_DECIM - 1) >= 5 * R) {          // this output reaches into the right neighbour's inputs
-                    const float rx = __shfl_down_sync(0xFFFFFFFFu, left[r].x, 1);
-                    const float ry = __shfl_down_sync(0xFFFFFFFFu, left[r].y, 1);
-                    own[r].x += rx;
-                    own[r].y += ry;
-                }
-            }
-            if (lane < 31) {
-#pragma unroll
-                for (int r = 0; r < R; r++) sm.yd[R * tq + r] = own[r];
-            }
-        }
-        __syncthreads();                                              // S1: xs[stage] consumed, yd complete
-        if (tid == 0 && use + 2 < n_tiles) {
-            unsigned s2 = s, it2 = it + 2;
-            if (it2 >= tiles_per_stream) it2 -= tiles_per_stream, s2++;
-            if (it2 >= tiles_per_stream) it2 -= tiles_per_stream, s2++;   // tiles_per_stream == 1
-            issue_tile<FMT>(sm, stage, p, tail8 + s2 * tail_bytes, iq8 + s2 * row_bytes, tile_l0(it2));
-        }
-
-        // ---- channel-select FIR: thread computes c[RC*tid .. RC*tid + RC), c[j] = sum_k h[k] * yd[j + 40 - k]
-        if (tid < C::NCT) {
-            float2 acc[C::RC];
-#pragma unroll
-            for (int r = 0; r < C::RC; r++) acc[r] = make_float2(dc, dc);
-            const float4* src = reinterpret_cast<const float4*>(&sm.yd[C::RC * tid]);
-#pragma unroll
-            for (int i = 0; i < (C::HC + C::RC) / 2; i++) {
-                const float4 v = src[i];
-                const float2 xa = make_float2(v.x, v.y), xb = make_float2(v.z, v.w);
-#pragma unroll
-                for (int r = 0; r < C::RC; r++) {
-                    const int ka = C::HC - 2 * i + r, kb = ka - 1;
-                    if (ka >= 0 && ka <= C::HC) acc[r] = cfma(c_taps_chan[ka], xa, acc[r]);
-                    if (kb >= 0 && kb <= C::HC) acc[r] = cfma(c_taps_chan[kb], xb, acc[r]);
-                }
-            }
-            float4* dst = reinterpret_cast<float4*>(&sm.c[C::RC * tid]);
-#pragma unroll
-            for (int r = 0; r < C::RC / 2; r++) dst[r] = make_float4(acc[2 * r].x, acc[2 * r].y, acc[2 * r + 1].x, acc[2 * r + 1].y);
-        }
-        __syncthreads();                                              // S2
-
-        // ---- FM discriminator, 4 per thread: d[j] from c[j + 1], c[j]; c[j] is output m_lo - 10 + j
-        float pw = 0.f;
-        const bool want_pw = p.power_sum != nullptr;
-        for (int q = tid; q < (C::ND + 3) / 4; q += C::NT) {
-            const int j0 = 4 * q;
-            const float4* src = reinterpret_cast<const float4*>(&sm.c[j0]);
-            const float4 v0 = src[0], v1 = src[1];
-            const float2 c4 = sm.c[j0 + 4];
-            const float2 cc[5] = {make_float2(v0.x, v0.y), make_float2(v0.z, v0.w), make_float2(v1.x, v1.y), make_float2(v1.z, v1.w), c4};
-            float dd[4];
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                const float2 prv = cc[i], cur = cc[i + 1];
-                const float re = cur.x * prv.x + cur.y * prv.y;
-                const float im = cur.y * prv.x - cur.x * prv.y;
-                dd[i] = disc_atan2(im, re) * P25_FM_GAIN;
-                const int o = j0 + i + 1 - P25_BOXCAR;                // stored-output index of c[j + 1]
-                if (want_pw && o >= 0 && o < nv) pw += cur.x * cur.x + cur.y * cur.y;
-            }
-            *reinterpret_cast<float4*>(&sm.d[j0]) = make_float4(dd[0], dd[1], dd[2], dd[3]);
-        }
-        __syncthreads();                                              // S3
-
-        // ---- symbol-period boxcar, 4 outputs per thread: out[o] = mean(d[o .. o + 9]), oldest first
-        for (int o0 = 4 * tid; o0 < nv; o0 += 4 * C::NT) {
-            const float4* src = reinterpret_cast<const float4*>(&sm.d[o0]);
-            const float4 a = src[0], b = src[1], c4 = src[2], e = src[3];
-            float s0 = a.x + a.y;
-            s0 += a.z; s0 += a.w; s0 += b.x; s0 += b.y; s0 += b.z; s0 += b.w; s0 += c4.x; s0 += c4.y;
-            const float s1 = (s0 - a.x) + c4.z, s2 = (s1 - a.y) + c4.w, s3 = (s2 - a.z) + e.x;
-            const float k = 1.0f / P25_BOXCAR;
-            float* out = p.bb + (size_t)s * p.row_stride + P25CU_BB_HIST + m_rel + o0;
-            if (o0 + 1 < nv) *reinterpret_cast<float2*>(out) = make_float2(s0 * k, s1 * k);
-            else out[0] = s0 * k;
-            if (o0 + 3 < nv) *reinterpret_cast<float2*>(out + 2) = make_float2(s2 * k, s3 * k);
-            else if (o0 + 2 < nv) out[2] = s2 * k;
-        }
-        if (p.power_sum) {
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) pw += __shfl_xor_sync(0xFFFFFFFFu, pw, o);
-            if (lane == 0) atomicAdd(p.power_sum + s, pw * pw_scale);
-        }
-        if (it == tiles_per_stream - 1) {   // last tile of the stream's chunk: carry the raw input tail (n >= HT here)
-            const uint4* src = reinterpret_cast<const uint4*>(iq8 + s * row_bytes + ((size_t)p.n - p.ht) * C::ES);
-            uint4* dst = reinterpret_cast<uint4*>((unsigned char*)p.tail_out + s * tail_bytes);
-            for (int i = tid; i < (int)(tail_bytes / 16); i += C::NT) dst[i] = src[i];
-        }
-        // no barrier needed here: the next tile's first shared-memory writes (yd) are two barriers away from
-        // the last reads of yd, and its d / c writes come after S1 / S2 of the next iteration
-        if (++it == tiles_per_stream) it = 0, s++;
-    }
-}
-
-}  // namespace fast5
+}  // namespace fast
 
 
 // =====================================================================================================
-// Warp-autonomous variant of the /5 fast path for u8 input (the reference's own format, where the FP32 pipe and
-// the issue slots, not HBM, are the limit).  The tile kernel above spends a third of its stall samples at CTA
-// barriers whose stages keep only part of the CTA busy; here every warp is its own pipeline and the only
+// /5 fast path for cf32 input (the reference's own chain at 240 kS/s; 16-byte aligned rows).  The FP32 pipe and the
+// issue slots, not HBM, are the limit of this shape (62 complex-by-real taps per 48 kHz output), and CTA barriers
+// between stages that keep only part of a CTA busy would stall both, so every warp is its own pipeline and the only
 // synchronisation is __syncwarp:
 //   * a warp walks a contiguous share of the flattened (stream, iteration) space, 124 outputs per iteration
 //     (31 lanes x 4; lane 31 only contributes its inputs' partial sums to lane 30), entering each stream or
 //     share with one discarded warm-up iteration, so the carried FIR histories live in per-warp shared memory;
-//   * lane 0 streams the raw 1.3 KB input slices with TMA bulk copies into a per-warp two-stage ring;
+//   * lane 0 streams the raw 5.1 KB input slices with TMA bulk copies into a per-warp two-stage ring;
+//   * decimator: a lane owns 20 consecutive inputs and forms its four outputs' own part plus the part it contributes
+//     to its left neighbour's last outputs, which neighbours exchange by warp shuffle (25 FFMA2 per output);
 //   * decimator outputs are kept as rows of four (two 16-byte halves in two arrays): a lane's 44-sample channel
 //     filter window is then 22 conflict-free LDS.128 of consecutive rows;
 //   * the channel filter's four outputs stay in registers for the discriminator (the previous sample arrives
@@ -1019,69 +746,33 @@ using fast::mbar_init;
 using fast::mbar_expect_tx;
 using fast::mbar_wait;
 using fast::tma_load_1d;
-using fast5::add2;
-using fast5::disc_atan2_pair;
-using fast5::load_u8;
+using fast::add2;
+using fast::disc_atan2_pair;
 
 constexpr int R = 4;                        // outputs per lane
 constexpr int NOUT = 31 * R;                // 124 outputs per warp iteration
 constexpr int XNEW = 5 * NOUT;              // 620 fresh input samples per iteration
 constexpr int XN = 32 * 5 * R;              // 640 samples read (the ghost lane's 20 included)
 constexpr int WARPS = 4;                    // per CTA
-template <int FMT>
-struct Fmt {                                // u8: 1.4 KB slices, 5 CTAs/SM; cf32: 5.1 KB slices, 4 CTAs/SM
-    static constexpr bool U8 = FMT == P25CU_FMT_U8_IQ;
-    static constexpr int AL = U8 ? 8 : 2, ES = U8 ? 2 : 8;
-    static constexpr int XLEN = (XN + 2 * AL - 2) / AL * AL;
-    static constexpr int XBYTES = (XLEN * ES + 127) / 128 * 128;
-    static constexpr int MINB = U8 ? 5 : 4;
-};
+constexpr int AL = 2, ES = 8;               // samples per 16 bytes, bytes per sample
+constexpr int XLEN = (XN + 2 * AL - 2) / AL * AL;
+constexpr int XBYTES = (XLEN * ES + 127) / 128 * 128;   // 5.1 KB slices
+constexpr int MINB = 4;                     // CTAs per SM
 constexpr int HROWS = (P25_TAPS_CHAN - 1) / R;        // 10 history rows of the decimator output
 constexpr int DROWS = 3;                    // history rows of the discriminator output (>= 9 samples)
 static_assert((P25_TAPS_CHAN - 1) % R == 0 && DROWS * R >= P25_BOXCAR - 1, "history rows");
 
-template <int FMT, bool MMA = false>
 struct __align__(128) WarpSm {
-    unsigned char xs[2][Fmt<FMT>::XBYTES];
+    unsigned char xs[2][XBYTES];
     float4 ydA[HROWS + 32], ydB[HROWS + 32];    // row i: (yd[4i], yd[4i+1]) | (yd[4i+2], yd[4i+3])
     float4 d4[DROWS + 32];
     unsigned long long full[2];
 };
 
-// Tensor-pipe variant of the channel filter (A/B switch P25CU_DDC5 bit 2; VERDICT r1 item 4 asked for a measurement,
-// not an estimate).  c[j] = sum_k h[k] y[j + 40 - k] over a block of 16 outputs is a [16 x 56] Toeplitz matrix times the
-// block's 56-sample window: seven mma.sync m16n8k8 TF32 steps whose eight columns are (four blocks) x (re, im).  FP32
-// accuracy comes from the split y = hi + lo, h = hi + lo with three products per step (hi hi, hi lo, lo hi; the error
-// is ~2^-21 relative).  The FIR leaves the FP32 pipe (41 of the 66 FFMA2 per output) for the legacy tensor pipe, which
-// pipe_peaks.cu measured at 476 TF32 MAC/clk/SM running beside FFMA2 at 80 % of its own peak.
-//   decimator outputs: two planes (re | im), window index i (0..39 history, 40..163 this iteration, 164..167 ghost)
-//   stored at i + 4 (i >> 4): every B-fragment load (8 columns x 4 rows) then hits 32 different banks.
-constexpr int YPLANE = 208;                     // 168 + 4 * 10 padded window samples per plane; 208 mod 32 = 16
-constexpr int CPAD = 160;                       // channel-filter outputs, o + 4 (o >> 4)
-__device__ __forceinline__ int ypad(int i) { return i + 4 * (i >> 4); }
-template <int FMT>
-struct __align__(128) WarpSm<FMT, true> {
-    unsigned char xs[2][Fmt<FMT>::XBYTES];
-    float y[2][YPLANE];
-    float2 c[CPAD];
-    float4 d4[DROWS + 32];
-    unsigned long long full[2];
-};
-constexpr int ATAB_FLOATS = 7 * 2 * 32 * 4;     // [k-step][hi | lo][lane][a0..a3]
-
-__device__ __forceinline__ void mma_tf32(float (&d)[4], const float4 a, const float b0, const float b1) {
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-                 : "r"(__float_as_uint(a.x)), "r"(__float_as_uint(a.y)), "r"(__float_as_uint(a.z)), "r"(__float_as_uint(a.w)),
-                   "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
-}
-
 // bulk copy of the slice whose first input has logical index l0 (tail ++ chunk); 32-bit index arithmetic, the slice
 // that still overlaps the carried tail (first iterations of a chunk only) takes the two-copy path
-template <int FMT, bool MMA>
-__device__ __forceinline__ void issue_slice(WarpSm<FMT, MMA>& sm, int stage, int ht, int lend, const unsigned char* tail,
+__device__ __forceinline__ void issue_slice(WarpSm& sm, int stage, int ht, int lend, const unsigned char* tail,
                                             const unsigned char* chunk, int l0) {
-    constexpr int AL = Fmt<FMT>::AL, ES = Fmt<FMT>::ES, XLEN = Fmt<FMT>::XLEN;
     const int la = l0 & ~(AL - 1);
     const int lb = min(la + XLEN, lend);
     if (la >= ht) {
@@ -1097,39 +788,17 @@ __device__ __forceinline__ void issue_slice(WarpSm<FMT, MMA>& sm, int stage, int
     if (nc) tma_load_1d(&sm.xs[stage][nt * ES], chunk, nc * ES, &sm.full[stage]);
 }
 
-template <int FMT, bool MMA>
-__global__ void __launch_bounds__(32 * WARPS, Fmt<FMT>::MINB) p25_ddc5_warp_kernel(const DdcParams p, const unsigned its_per_stream,
-                                                                             const float dc, const float pw_scale) {
-    constexpr int AL = Fmt<FMT>::AL, ES = Fmt<FMT>::ES;
+__global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_warp_kernel(const DdcParams p, const unsigned its_per_stream,
+                                                                         const float dc, const float pw_scale) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    WarpSm<FMT, MMA>& sm = reinterpret_cast<WarpSm<FMT, MMA>*>(smem_raw)[warp];
+    WarpSm& sm = reinterpret_cast<WarpSm*>(smem_raw)[warp];
     if (lane == 0) {
         mbar_init(&sm.full[0], 1);
         mbar_init(&sm.full[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    [[maybe_unused]] const float4* atab = nullptr;
-    if constexpr (MMA) {
-        // Toeplitz A fragments of the seven k-steps, split into TF32 hi and lo parts, built once per CTA:
-        // A[i][kk] = h[40 + i - kk] (output row i of the block, window position kk), zero outside the band
-        float* at = reinterpret_cast<float*>(smem_raw + sizeof(WarpSm<FMT, true>) * WARPS);
-        for (int e = threadIdx.x; e < ATAB_FLOATS / 2; e += 32 * WARPS) {
-            const int q = e & 3, ln = (e >> 2) & 31, st = e >> 7;
-            const int row = (ln >> 2) + ((q & 1) ? 8 : 0), kk = 8 * st + (ln & 3) + ((q & 2) ? 4 : 0);
-            const int k = (P25_TAPS_CHAN - 1) + row - kk;
-            const float h = (k >= 0 && k < P25_TAPS_CHAN) ? c_taps_chan[k] : 0.f;
-            const float hi = __uint_as_float(__float_as_uint(h) & 0xFFFFE000u);
-            at[(st * 2 + 0) * 128 + ln * 4 + q] = hi;
-            at[(st * 2 + 1) * 128 + ln * 4 + q] = h - hi;
-        }
-        atab = reinterpret_cast<const float4*>(at);
-        for (int i = lane; i < 2 * YPLANE; i += 32) (&sm.y[0][0])[i] = 0.f;
-        for (int i = lane; i < CPAD; i += 32) sm.c[i] = make_float2(0.f, 0.f);
-        __syncthreads();
-    } else {
-        for (int i = lane; i < HROWS + 32; i += 32) sm.ydA[i] = sm.ydB[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
+    for (int i = lane; i < HROWS + 32; i += 32) sm.ydA[i] = sm.ydB[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int i = lane; i < DROWS + 32; i += 32) sm.d4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     __syncwarp();
 
@@ -1150,8 +819,8 @@ __global__ void __launch_bounds__(32 * WARPS, Fmt<FMT>::MINB) p25_ddc5_warp_kern
     const unsigned char* chunk = (const unsigned char*)p.iq + s * row_bytes;
     const unsigned char* tail = (const unsigned char*)p.tail_in + s * tail_bytes;
     if (lane == 0) {                                        // warm-up and first stored iteration of the first piece
-        issue_slice<FMT, MMA>(sm, 0, ht, lend, tail, chunk, l_base + XNEW * (it_first - 1));
-        issue_slice<FMT, MMA>(sm, 1, ht, lend, tail, chunk, l_base + XNEW * it_first);
+        issue_slice(sm, 0, ht, lend, tail, chunk, l_base + XNEW * (it_first - 1));
+        issue_slice(sm, 1, ht, lend, tail, chunk, l_base + XNEW * it_first);
     }
     float2 c_carry = make_float2(0.f, 0.f);
     unsigned use = 0;
@@ -1169,32 +838,26 @@ __global__ void __launch_bounds__(32 * WARPS, Fmt<FMT>::MINB) p25_ddc5_warp_kern
         const int nv = j ? min(n_out - NOUT * it, NOUT) : 0;     // j = 0 is the warm-up: nothing is stored
         mbar_wait(&sm.full[stage], (use >> 1) & 1);
 
-        // ---- /5 decimator (same arithmetic as the tile kernel): lane owns inputs [20 lane, 20 lane + 20)
+        // ---- /5 decimator: lane owns inputs [20 lane, 20 lane + 20)
         float2 own[R];
         {
             float2 x[5 * R];
             const int s0 = skew + 5 * R * lane;
-            if constexpr (Fmt<FMT>::U8) {
-                const unsigned* wp = reinterpret_cast<const unsigned*>(sm.xs[stage]) + (s0 >> 1);
-                if (s0 & 1) load_u8<R, true>(wp, x);
-                else load_u8<R, false>(wp, x);
+            // 16-byte loads (two samples): half the wavefronts of LDS.64 at this 160-byte lane stride
+            const float4* xp = reinterpret_cast<const float4*>(reinterpret_cast<const float2*>(sm.xs[stage]) + (s0 & ~1));
+            if (s0 & 1) {
+#pragma unroll
+                for (int i = 0; i <= 5 * R / 2; i++) {
+                    const float4 v = xp[i];
+                    if (i > 0) x[2 * i - 1] = make_float2(v.x, v.y);
+                    if (i < 5 * R / 2) x[2 * i] = make_float2(v.z, v.w);
+                }
             } else {
-                // 16-byte loads (two samples): half the wavefronts of LDS.64 at this 160-byte lane stride
-                const float4* xp = reinterpret_cast<const float4*>(reinterpret_cast<const float2*>(sm.xs[stage]) + (s0 & ~1));
-                if (s0 & 1) {
 #pragma unroll
-                    for (int i = 0; i <= 5 * R / 2; i++) {
-                        const float4 v = xp[i];
-                        if (i > 0) x[2 * i - 1] = make_float2(v.x, v.y);
-                        if (i < 5 * R / 2) x[2 * i] = make_float2(v.z, v.w);
-                    }
-                } else {
-#pragma unroll
-                    for (int i = 0; i < 5 * R / 2; i++) {
-                        const float4 v = xp[i];
-                        x[2 * i] = make_float2(v.x, v.y);
-                        x[2 * i + 1] = make_float2(v.z, v.w);
-                    }
+                for (int i = 0; i < 5 * R / 2; i++) {
+                    const float4 v = xp[i];
+                    x[2 * i] = make_float2(v.x, v.y);
+                    x[2 * i + 1] = make_float2(v.z, v.w);
                 }
             }
             float2 lft[R];
@@ -1218,65 +881,16 @@ __global__ void __launch_bounds__(32 * WARPS, Fmt<FMT>::MINB) p25_ddc5_warp_kern
                 }
             }
         }
-        if constexpr (MMA) {                       // window index 40 + 4 lane + r, re and im planes (lane 31: finite ghost values)
-            const int pi = ypad(4 * HROWS + R * lane);
-            *reinterpret_cast<float4*>(&sm.y[0][pi]) = make_float4(own[0].x, own[1].x, own[2].x, own[3].x);
-            *reinterpret_cast<float4*>(&sm.y[1][pi]) = make_float4(own[0].y, own[1].y, own[2].y, own[3].y);
-        } else {
-            sm.ydA[HROWS + lane] = make_float4(own[0].x, own[0].y, own[1].x, own[1].y);   // lane 31's row is never read
-            sm.ydB[HROWS + lane] = make_float4(own[2].x, own[2].y, own[3].x, own[3].y);
-        }
+        sm.ydA[HROWS + lane] = make_float4(own[0].x, own[0].y, own[1].x, own[1].y);   // lane 31's row is never read
+        sm.ydB[HROWS + lane] = make_float4(own[2].x, own[2].y, own[3].x, own[3].y);
         __syncwarp();                                                                 // S1: xs[stage] consumed, rows visible
         if (lane == 0) {                                    // prefetch two iterations ahead (possibly into the next piece)
-            if (j + 2 < npiece) issue_slice<FMT, MMA>(sm, stage, ht, lend, tail, chunk, l_base + XNEW * (it + 2));
-            else if (left) issue_slice<FMT, MMA>(sm, stage, ht, lend, tail + tail_bytes, chunk + row_bytes, l_base + XNEW * (j + 1 - npiece));
+            if (j + 2 < npiece) issue_slice(sm, stage, ht, lend, tail, chunk, l_base + XNEW * (it + 2));
+            else if (left) issue_slice(sm, stage, ht, lend, tail + tail_bytes, chunk + row_bytes, l_base + XNEW * (j + 1 - npiece));
         }
 
-        float2 acc[R];
-        if constexpr (MMA) {
-            // ---- channel-select FIR on the tensor pipe: two D tiles (blocks 0..3 | 4..7) x seven k-steps x three products
-            const int g = lane >> 2, tig = lane & 3;
-            const float* yp = &sm.y[g & 1][0];                       // column n = g: block (g >> 1) of the tile, component g & 1
-            float d0[4] = {dc, dc, dc, dc}, d1[4] = {dc, dc, dc, dc};
-#pragma unroll
-            for (int st = 0; st < 7; st++) {
-                const float4 ah = atab[(2 * st) * 32 + lane], al = atab[(2 * st + 1) * 32 + lane];
-#pragma unroll
-                for (int t = 0; t < 2; t++) {
-                    const int i0 = 16 * (4 * t + (g >> 1)) + 8 * st + tig;      // window sample of B row tig; row tig + 4 is i0 + 4
-                    const float b0 = yp[ypad(i0)], b1 = yp[ypad(i0 + 4)];
-                    const float b0h = __uint_as_float(__float_as_uint(b0) & 0xFFFFE000u), b1h = __uint_as_float(__float_as_uint(b1) & 0xFFFFE000u);
-                    const float b0l = b0 - b0h, b1l = b1 - b1h;
-                    if (t == 0) {
-                        mma_tf32(d0, ah, b0h, b1h);
-                        mma_tf32(d0, ah, b0l, b1l);
-                        mma_tf32(d0, al, b0h, b1h);
-                    } else {
-                        mma_tf32(d1, ah, b0h, b1h);
-                        mma_tf32(d1, ah, b0l, b1l);
-                        mma_tf32(d1, al, b0h, b1h);
-                    }
-                }
-            }
-            // D fragment: (d[0], d[1]) = (re, im) of output 16 (4 t + tig) + g, (d[2], d[3]) of that output + 8
-            {
-                const int o0 = 16 * tig + g, o1 = 64 + 16 * tig + g;
-                sm.c[ypad(o0)] = make_float2(d0[0], d0[1]);
-                sm.c[ypad(o0 + 8)] = make_float2(d0[2], d0[3]);
-                sm.c[ypad(o1)] = make_float2(d1[0], d1[1]);
-                sm.c[ypad(o1 + 8)] = make_float2(d1[2], d1[3]);
-            }
-            __syncwarp();
-            {
-                const float4* cp = reinterpret_cast<const float4*>(&sm.c[ypad(R * lane)]);
-                const float4 v0 = cp[0], v1 = cp[1];
-                acc[0] = make_float2(v0.x, v0.y);
-                acc[1] = make_float2(v0.z, v0.w);
-                acc[2] = make_float2(v1.x, v1.y);
-                acc[3] = make_float2(v1.z, v1.w);
-            }
-        } else {
         // ---- channel-select FIR: outputs 4 lane + r, window = rows lane .. lane + 10 (44 samples, s = 40 + r - k)
+        float2 acc[R];
 #pragma unroll
         for (int r = 0; r < R; r++) acc[r] = make_float2(dc, dc);
 #pragma unroll
@@ -1291,7 +905,6 @@ __global__ void __launch_bounds__(32 * WARPS, Fmt<FMT>::MINB) p25_ddc5_warp_kern
                     if (k >= 0 && k < P25_TAPS_CHAN) acc[r] = cfma(c_taps_chan[k], xs4[q], acc[r]);
                 }
             }
-        }
         }
         // ---- FM discriminator on the four outputs in registers; the sample before comes from the lane below
         float2 prev;
@@ -1338,20 +951,13 @@ __global__ void __launch_bounds__(32 * WARPS, Fmt<FMT>::MINB) p25_ddc5_warp_kern
         }
         // ---- roll the histories: the last 10 decimator rows and 3 discriminator rows move to the front
         float4 ra = make_float4(0.f, 0.f, 0.f, 0.f), rb = ra, rd = ra;
-        if constexpr (MMA) {                       // window samples 124 .. 163 -> 0 .. 39 in both planes (padded indices differ)
-            if (lane < 20) {
-                const int src = NOUT + 4 * (lane >> 1), pl = lane & 1;
-                ra = make_float4(sm.y[pl][ypad(src)], sm.y[pl][ypad(src + 1)], sm.y[pl][ypad(src + 2)], sm.y[pl][ypad(src + 3)]);
-            }
-        } else if (lane < HROWS) {
+        if (lane < HROWS) {
             ra = sm.ydA[31 + lane];
             rb = sm.ydB[31 + lane];
         }
         if (lane < DROWS) rd = sm.d4[31 + lane];
         __syncwarp();                                                                 // S3
-        if constexpr (MMA) {
-            if (lane < 20) *reinterpret_cast<float4*>(&sm.y[lane & 1][ypad(4 * (lane >> 1))]) = ra;
-        } else if (lane < HROWS) {
+        if (lane < HROWS) {
             sm.ydA[lane] = ra;
             sm.ydB[lane] = rb;
         }
@@ -1381,8 +987,9 @@ __global__ void __launch_bounds__(32 * WARPS, Fmt<FMT>::MINB) p25_ddc5_warp_kern
 
 // =====================================================================================================
 // /5 warp kernel for u8 input with the DECIMATOR ON THE INTEGER TENSOR PIPE (round 2; VERDICT r1 item 4: "integer-domain
-// decimator on the raw bytes").  The warp kernel above is bound by the FP32 pipe: 21 of its 62 FIR FFMA2 per output are
-// the /5 decimator, and every input byte costs two PRMT + half a FADD2 before it can enter an FFMA2.  Here the raw bytes
+// decimator on the raw bytes").  On FFMA2 alone (the warp kernel above) the /5 chain is bound by the FP32 pipe: 21 of its
+// 62 FIR FFMA2 per output are the /5 decimator, and every u8 input byte would cost two PRMT + half a FADD2 before it
+// could enter an FFMA2.  Here the raw bytes
 // go into mma.sync.m16n8k32.s32.u8.s8 as they lie in the TMA-staged slice, without any conversion:
 //   * A (16 x 32 bytes per k-step) = sixteen overlapping rows of the slice, row m starting 40 samples (80 bytes) after
 //     row m - 1, interleaved I/Q bytes along k; a row's 64-sample window holds the inputs of eight consecutive outputs;
@@ -1409,8 +1016,8 @@ using fast::mbar_expect_tx;
 using fast::mbar_wait;
 using fast::tma_load_1d;
 using fast::cfma;
-using fast5::add2;
-using fast5::disc_atan2_pair;
+using fast::add2;
+using fast::disc_atan2_pair;
 
 constexpr int R = 8;                                    // outputs per lane
 constexpr int NOUT = 32 * R;                            // 256 outputs per warp iteration: two m-tiles of 16 rows x 8 outputs
@@ -1724,8 +1331,8 @@ using fast::mbar_expect_tx;
 using fast::mbar_wait;
 using fast::tma_load_1d;
 using fast::cfma;
-using fast5::add2;
-using fast5::disc_atan2_pair;
+using fast::add2;
+using fast::disc_atan2_pair;
 using w5i::imma;
 using w5i::imma0;
 using w5i::lds32;
@@ -2053,34 +1660,14 @@ static cudaError_t launch_fast(const DdcParams& p, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-template <int FMT>
-static cudaError_t launch_fast5(const DdcParams& p, cudaStream_t st) {
-    using C = fast5::K<FMT>;
-    auto kern = fast5::p25_ddc5_fm_kernel<FMT>;
-    const size_t smem = sizeof(fast5::Smem<FMT>);
-    const int grid_max = p.plan->grid_fast5[FMT];
-    const unsigned tps = (p.n_out + C::MB - 1) / C::MB;
-    const unsigned long long total = (unsigned long long)p.n_streams * tps;
-    const unsigned grid = total < (unsigned long long)grid_max ? (unsigned)total : (unsigned)grid_max;
-    const float dc = C::U8 ? (float)(0.5 * tap_gain(P25_TAPS_DECIM_H, P25_TAPS_DECIM) * tap_gain(P25_TAPS_CHAN_H, P25_TAPS_CHAN)) : 0.f;
-    const float pw_scale = C::U8 ? (float)(1.0 / (127.5 * 127.5)) : 1.f;
-    kern<<<grid, C::NT, smem, st>>>(p, tps, dc, pw_scale);
-    return cudaGetLastError();
-}
-
-template <int FMT, bool MMA>
 static cudaError_t launch_w5(const DdcParams& p, cudaStream_t st) {
-    auto kern = w5::p25_ddc5_warp_kernel<FMT, MMA>;
-    const size_t smem = sizeof(w5::WarpSm<FMT, MMA>) * w5::WARPS + (MMA ? w5::ATAB_FLOATS * sizeof(float) : 0);
-    const int grid_max = MMA ? p.plan->grid_w5m[FMT] : p.plan->grid_w5[FMT];
+    const size_t smem = sizeof(w5::WarpSm) * w5::WARPS;
     const unsigned ips = (p.n_out + w5::NOUT - 1) / w5::NOUT;
     const unsigned long long total = (unsigned long long)p.n_streams * ips;
     unsigned long long want = (total + 3) / 4;                 // at least ~4 iterations per warp (one warm-up each)
     want = (want + w5::WARPS - 1) / w5::WARPS;
-    const unsigned grid = want < (unsigned long long)grid_max ? (unsigned)(want ? want : 1) : (unsigned)grid_max;
-    const bool u8 = FMT == P25CU_FMT_U8_IQ;
-    const float dc = u8 ? (float)(0.5 * tap_gain(P25_TAPS_DECIM_H, P25_TAPS_DECIM) * tap_gain(P25_TAPS_CHAN_H, P25_TAPS_CHAN)) : 0.f;
-    kern<<<grid, 32 * w5::WARPS, smem, st>>>(p, ips, dc, u8 ? (float)(1.0 / (127.5 * 127.5)) : 1.f);
+    const unsigned grid = want < (unsigned long long)p.plan->grid_w5 ? (unsigned)(want ? want : 1) : (unsigned)p.plan->grid_w5;
+    w5::p25_ddc5_warp_kernel<<<grid, 32 * w5::WARPS, smem, st>>>(p, ips, 0.f, 1.f);
     return cudaGetLastError();
 }
 
@@ -2136,31 +1723,13 @@ cudaError_t p25cu_ddc_plan_device(P25DevPlan* plan) {
     constexpr int U8 = P25CU_FMT_U8_IQ, CF = P25CU_FMT_CF32_IQ;
     if ((e = plan_one(fast::p25_ddc_fm_stream_kernel<CF>, fast::NT, sizeof(fast::Smem<CF>), n_sm, &plan->grid_ddc50)) != cudaSuccess) return e;
     if ((e = plan_one(fast::p25_ddc_fm_stream_kernel<U8>, fast::NT, sizeof(fast::Smem<U8>), n_sm, &plan->grid_ddc50_u8)) != cudaSuccess) return e;
-    if (const char* ev = getenv("P25CU_DDC_CTAS")) {   // A/B: CTAs per SM of the persistent /50 grids
-        const int per_sm = atoi(ev);
-        if (per_sm > 0) plan->grid_ddc50 = plan->grid_ddc50_u8 = n_sm * per_sm;
-    }
-    if ((e = plan_one(fast5::p25_ddc5_fm_kernel<U8>, fast5::K<U8>::NT, sizeof(fast5::Smem<U8>), n_sm, &plan->grid_fast5[U8])) != cudaSuccess) return e;
-    if ((e = plan_one(fast5::p25_ddc5_fm_kernel<CF>, fast5::K<CF>::NT, sizeof(fast5::Smem<CF>), n_sm, &plan->grid_fast5[CF])) != cudaSuccess) return e;
-    if ((e = plan_one(w5::p25_ddc5_warp_kernel<U8, false>, 32 * w5::WARPS, sizeof(w5::WarpSm<U8>) * w5::WARPS, n_sm, &plan->grid_w5[U8])) != cudaSuccess) return e;
-    if ((e = plan_one(w5::p25_ddc5_warp_kernel<CF, false>, 32 * w5::WARPS, sizeof(w5::WarpSm<CF>) * w5::WARPS, n_sm, &plan->grid_w5[CF])) != cudaSuccess) return e;
-    if (const char* ev = getenv("P25CU_W5_CTAS")) {    // A/B: CTAs per SM of the persistent /5 warp-kernel grids
-        const int per_sm = atoi(ev);
-        if (per_sm > 0) plan->grid_w5[U8] = plan->grid_w5[CF] = n_sm * per_sm;
-    }
+    if ((e = plan_one(w5::p25_ddc5_warp_kernel, 32 * w5::WARPS, sizeof(w5::WarpSm) * w5::WARPS, n_sm, &plan->grid_w5)) != cudaSuccess) return e;
     const size_t smem_w5i = sizeof(w5i::WarpSm) * w5i::WARPS + sizeof(uint2) * w5i::NB * 32;
     if ((e = plan_one(w5i::p25_ddc5_imma_kernel<true>, 32 * w5i::WARPS, smem_w5i, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
     if ((e = plan_one(w5i::p25_ddc5_imma_kernel<false>, 32 * w5i::WARPS, smem_w5i, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
-    if (const char* ev = getenv("P25CU_W5_CTAS")) {
-        const int per_sm = atoi(ev);
-        if (per_sm > 0) plan->grid_w5i = n_sm * per_sm;
-    }
     const size_t smem_w50i = sizeof(w50i::WarpSm) * w50i::WARPS + sizeof(uint2) * w50i::NB * 32;
     if ((e = plan_one(w50i::p25_ddc50_imma_kernel<true>, 32 * w50i::WARPS, smem_w50i, n_sm, &plan->grid_w50i)) != cudaSuccess) return e;
     if ((e = plan_one(w50i::p25_ddc50_imma_kernel<false>, 32 * w50i::WARPS, smem_w50i, n_sm, &plan->grid_w50i)) != cudaSuccess) return e;
-    const size_t atab = w5::ATAB_FLOATS * sizeof(float);
-    if ((e = plan_one(w5::p25_ddc5_warp_kernel<U8, true>, 32 * w5::WARPS, sizeof(w5::WarpSm<U8, true>) * w5::WARPS + atab, n_sm, &plan->grid_w5m[U8])) != cudaSuccess) return e;
-    if ((e = plan_one(w5::p25_ddc5_warp_kernel<CF, true>, 32 * w5::WARPS, sizeof(w5::WarpSm<CF, true>) * w5::WARPS + atab, n_sm, &plan->grid_w5m[CF])) != cudaSuccess) return e;
     // the generic kernels' shared memory (27 - 72 KB) needs the opt-in as well
     if ((e = cudaFuncSetAttribute(p25_ddc_fm_kernel<true, U8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem<true>))) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(p25_ddc_fm_kernel<true, CF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem<true>))) != cudaSuccess) return e;
@@ -2168,35 +1737,20 @@ cudaError_t p25cu_ddc_plan_device(P25DevPlan* plan) {
     return cudaFuncSetAttribute(p25_ddc_fm_kernel<false, CF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem<false>));
 }
 
-// /5 fast paths: bit 0 = warp-autonomous kernel for u8, bit 1 = for cf32 (otherwise the tile kernel), bit 2 = its channel
-// filter on the tensor pipe, bit 3 = u8 warp kernel with the decimator on the integer tensor pipe; A/B switch P25CU_DDC5
-static int ddc5_variant() {
-    static const int v = getenv("P25CU_DDC5") ? atoi(getenv("P25CU_DDC5")) : 11;
-    return v;
-}
-
 cudaError_t p25cu_launch_ddc(const DdcParams& p, int format, int decimation, cudaStream_t st) {
     if (p.n_out == 0 && p.n == 0) return cudaSuccess;
-    if (decimation == 5 && p.aligned16 && p.n_out > 0 && p.a0 >= p.ht && p.n >= p.ht && p.ht == (unsigned)Cfg<false>::HT) {
-        const bool mma = (ddc5_variant() & 4) != 0;     // channel filter on the tensor pipe (mma.sync 3xTF32)
-        if (format == P25CU_FMT_U8_IQ && (ddc5_variant() & 8)) return launch_w5i(p, st);   // decimator on the integer tensor pipe
-        if (format == P25CU_FMT_U8_IQ && (ddc5_variant() & 1))
-            return mma ? launch_w5<P25CU_FMT_U8_IQ, true>(p, st) : launch_w5<P25CU_FMT_U8_IQ, false>(p, st);
-        if (format == P25CU_FMT_CF32_IQ && (ddc5_variant() & 2))
-            return mma ? launch_w5<P25CU_FMT_CF32_IQ, true>(p, st) : launch_w5<P25CU_FMT_CF32_IQ, false>(p, st);
-    }
-    // /5 fast path: aligned rows, the whole history inside the stream (no implicit zeros), chunk at least one tail long
+    // /5 fast paths: aligned rows, the whole history inside the stream (no implicit zeros), chunk at least one tail long
     if (decimation == 5 && p.aligned16 && p.n_out > 0 && p.a0 >= p.ht && p.n >= p.ht && p.ht == (unsigned)Cfg<false>::HT)
-        return format == P25CU_FMT_CF32_IQ ? launch_fast5<P25CU_FMT_CF32_IQ>(p, st) : launch_fast5<P25CU_FMT_U8_IQ>(p, st);
+        return format == P25CU_FMT_CF32_IQ ? launch_w5(p, st) : launch_w5i(p, st);
     if (decimation == 50 && format == P25CU_FMT_CF32_IQ && p.aligned16 && (p.a0 & 1ull) == 0 && p.n_out > 0 &&
         p.ht == (unsigned)Cfg<true>::HT)
         return launch_fast<P25CU_FMT_CF32_IQ>(p, st);
     // u8 at 2.4 MS/s: any decimator phase (blocks are staged from their enclosing 16-byte group); like the /5 fast paths the
     // whole history must lie inside the stream (no byte encodes the zeros in front of a stream start)
     if (decimation == 50 && format == P25CU_FMT_U8_IQ && p.aligned16 && p.n_out > 0 && p.a0 >= p.ht && p.ht == (unsigned)Cfg<true>::HT) {
-        // both decimating stages on the integer tensor pipe (A/B switch P25CU_DDC50: 0 = the FFMA2 stream kernel)
-        static const int v50 = getenv("P25CU_DDC50") ? atoi(getenv("P25CU_DDC50")) : 1;
-        if ((v50 & 1) && p.n >= p.ht) return launch_w50i(p, st);
+        // both decimating stages on the integer tensor pipe; it carries the tail from the chunk itself, so a chunk
+        // shorter than the tail takes the FFMA2 stream kernel
+        if (p.n >= p.ht) return launch_w50i(p, st);
         return launch_fast<P25CU_FMT_U8_IQ>(p, st);
     }
     if (decimation == 50)

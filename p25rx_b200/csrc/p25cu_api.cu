@@ -181,13 +181,11 @@ static int create_impl(p25cu_ctx* ctx) {
         }
         ctx->plan = &g_plans[cfg.device];
     }
-    {   // stream priorities (A/B switch P25CU_WALK_PRIO: 0 = demod first, 1 = walker first, 2 = equal)
+    {   // stream priorities: demod (stream) first, walker (stream2) last
         int lo = 0, hi = 0;
         CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        const char* e = getenv("P25CU_WALK_PRIO");
-        const int mode = e ? atoi(e) : 0;
-        CK(cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, mode == 1 ? lo : hi));
-        CK(cudaStreamCreateWithPriority(&ctx->stream2, cudaStreamNonBlocking, mode == 0 ? lo : hi));
+        CK(cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, hi));
+        CK(cudaStreamCreateWithPriority(&ctx->stream2, cudaStreamNonBlocking, lo));
         CK(cudaStreamCreateWithFlags(&ctx->stream_copy, cudaStreamNonBlocking));
     }
     for (int i = 0; i < 2; i++) {
@@ -200,7 +198,6 @@ static int create_impl(p25cu_ctx* ctx) {
     // The walker runs beside the next chunk's demod kernel only where that kernel is HBM-bound (cf32 /50: issue slots
     // are free); the u8 /50, /5 and channelizer kernels are issue-bound themselves and co-running only slows both (measured).
     ctx->overlap = (cfg.decimation == 50 && cfg.format == P25CU_FMT_CF32_IQ) ? 1 : 0;
-    if (const char* e = getenv("P25CU_OVERLAP")) ctx->overlap = atoi(e) ? 1 : 0;   // A/B switch
     ctx->walk_prefilter = cfg.decimation == (int)p25cu_pfb_decimation() ? 1 : 0;
     if (const char* e = getenv("P25CU_WALK_PREFILTER")) ctx->walk_prefilter = atoi(e) ? 1 : 0;   // A/B switch (same output either way)
     const size_t S = cfg.n_streams;
@@ -455,8 +452,8 @@ extern "C" int p25cu_decode(p25cu_ctx* ctx, const float* baseband, size_t n) {
     // 3 CTAs x 320 threads x 56 allocated registers per SM.  Two 64-thread walker CTAs fit in the registers that are
     // left (a third would keep a demod CTA from becoming resident: measured 0.51 vs 0.57 ms per step), so the walker
     // is launched as a persistent grid of 2 CTAs per SM that walks the streams in several passes.
-    static const int persist = getenv("P25CU_WALK_PERSIST") ? atoi(getenv("P25CU_WALK_PERSIST")) : 2;
-    CK(p25cu_launch_walk(w, ws, ctx->overlap && persist ? (unsigned)(ctx->n_sm * persist) : 0u, ctx->cfg.device, ctx->walk_prefilter != 0));
+    constexpr unsigned walk_ctas_per_sm = 2;
+    CK(p25cu_launch_walk(w, ws, ctx->overlap ? (unsigned)ctx->n_sm * walk_ctas_per_sm : 0u, ctx->cfg.device, ctx->walk_prefilter != 0));
     CK(cudaEventRecord(ctx->ev_bb_free[buf], ws));
     if (!ctx->overlap) CK(cudaStreamWaitEvent(ctx->stream2, ctx->ev_bb_free[buf], 0));   // keep stream2 consumers ordered
     ctx->launches++;

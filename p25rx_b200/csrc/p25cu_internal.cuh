@@ -84,9 +84,7 @@ struct P25DevPlan {
     int n_sm;
     int grid_ddc50;               // persistent grid of fast::p25_ddc_fm_stream_kernel
     int grid_ddc50_u8;            // ... of its u8 instantiation
-    int grid_fast5[2];            // fast5::p25_ddc5_fm_kernel<FMT>
-    int grid_w5[2];               // w5::p25_ddc5_warp_kernel<FMT, false>
-    int grid_w5m[2];              // ... with the channel filter on the tensor pipe
+    int grid_w5;                  // w5::p25_ddc5_warp_kernel (cf32 /5)
     int grid_w50i;                // w50i::p25_ddc50_imma_kernel (u8 /50, both decimating stages on the integer tensor pipe)
     int grid_w5i;                 // w5i::p25_ddc5_imma_kernel (u8, decimator on the integer tensor pipe)
     int pfb_slots;                // resident CTAs of the channelizer kernel

@@ -86,7 +86,7 @@ __device__ __forceinline__ void dft8(float2 (&v)[8]) {
     v[7] = csub(E3, T3);
 }
 
-__device__ __forceinline__ float atan2_branchfree(float y, float x) {   // same polynomial as ddc_fm.cu disc_atan2
+__device__ __forceinline__ float atan2_branchfree(float y, float x) {   // same polynomial as ddc_fm.cu disc_atan2_pair
     const float ax = fabsf(x), ay = fabsf(y);
     const float mx = fmaxf(ax, ay), mn = fminf(ax, ay);
     float rc;

@@ -12,21 +12,21 @@ sys.path.insert(0, os.path.join(ROOT, "spec"))
 
 from tools import p25tx as tx  # noqa: E402
 
-EXE = os.path.join(ROOT, "tests", "cpp", "p25host_main")
 
-
-def build_host_main():
+def build_host_main(out_dir):
+    """Link tests/cpp/p25host_main.cpp against the built library into out_dir: the source tree may be read-only."""
     lib_dir = os.path.join(ROOT, "p25rx_b200")
+    exe = os.path.join(str(out_dir), "p25host_main")
     subprocess.check_call(["g++", "-std=c++17", "-O2", "-Wall", "-Wextra", "-I", os.path.join(ROOT, "include"),
-                           os.path.join(ROOT, "tests", "cpp", "p25host_main.cpp"), "-o", EXE,
+                           os.path.join(ROOT, "tests", "cpp", "p25host_main.cpp"), "-o", exe,
                            "-L", lib_dir, "-lp25cu", f"-Wl,-rpath,{lib_dir}"])
-    return EXE
+    return exe
 
 
-def test_cpp_host_layer_compiles_and_links():
+def test_cpp_host_layer_compiles_and_links(tmp_path):
     import p25rx_b200
     p25rx_b200.build()
-    exe = build_host_main()
+    exe = build_host_main(tmp_path)
     r = subprocess.run([exe], capture_output=True, text=True)
     assert r.returncode == 2 and "usage" in r.stderr            # no GPU work without arguments
 
@@ -52,7 +52,7 @@ def _parse(out: str):
 def test_cpp_replay_receiver_matches_oracle(tmp_path):
     from oracle import pyoracle as po
     from p25rx_b200 import consumers as co
-    exe = build_host_main()
+    exe = build_host_main(tmp_path)
     paths, ref, ref_stats, n_voice = [], [], np.zeros((12, 4), dtype=np.uint64), 0
     po.lib().p25o_set_always_correlate(0)
     for s in range(3):
@@ -84,7 +84,7 @@ def test_cpp_replay_receiver_matches_oracle(tmp_path):
 @pytest.mark.gpu
 def test_cpp_demod_task_and_receiver_match_oracle(tmp_path):
     from oracle import pyoracle as po
-    exe = build_host_main()
+    exe = build_host_main(tmp_path)
     po.lib().p25o_set_always_correlate(0)
     paths, ref, ref_pw, n_chunks = [], [], {}, 6
     for s in range(2):
@@ -162,7 +162,7 @@ def _parse_consumer(out: str):
     return tg, hub
 
 
-def test_cpp_consumer_fields_match_python_adapters():
+def test_cpp_consumer_fields_match_python_adapters(tmp_path):
     """include/p25cu.hpp TsbkFields / LinkControlFields / fields:: / ChannelParamsMap / RecvConsumer against
     p25rx_b200/consumers.py on hand-built payloads (no GPU): talkgroups with their traffic-channel frequency and the
     hub's status JSON, including what must be dropped (bad CRC, manufacturer id, reserved talkgroups, unknown channel ids)."""
@@ -170,7 +170,7 @@ def test_cpp_consumer_fields_match_python_adapters():
     import p25rx_b200
     from p25rx_b200 import consumers as co
     p25rx_b200.build()
-    exe = build_host_main()
+    exe = build_host_main(tmp_path)
     ev, argv = _consumer_events()
     r = subprocess.run([exe, "fields"] + argv, capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
@@ -193,7 +193,7 @@ def test_cpp_consumer_view_of_decoded_streams(tmp_path):
     import json
     import p25rx_b200 as p25
     from p25rx_b200 import consumers as co
-    exe = build_host_main()
+    exe = build_host_main(tmp_path)
     tsbks, lcs = _consumer_units()
     units = []
     for i in range(0, len(tsbks), 3):

@@ -514,14 +514,16 @@ def test_channelizer_is_invariant_under_chunking(p25, oracle):
 # ------------------------------------------------------------------ integer-tensor-pipe decimators: chunk phases and edge sizes
 @pytest.mark.parametrize("dec,chunks", [
     (5, [16384, 1312, 1320, 2568, 5128, 20000, 1312, 8]),          # 1312 = the carried tail: the smallest fast-path chunk
-    (50, [16384, 3264, 3272, 6648, 12808, 40000, 3264, 8]),
+    (50, [16384, 3264, 3272, 6648, 12808, 40000, 3264, 8, 1608, 3264]),   # 1608: shorter than the tail
 ])
 def test_u8_imma_kernels_chunk_phases_and_minimal_chunks(p25, oracle, dec, chunks):
     """w5i / w50i (u8, decimator stages as u8 x s8 mma.sync on the raw bytes): a chunk sequence that walks the slice's
     alignment inside its 16-byte group through every value it can take, with chunks as short as the carried tail (one warp
     iteration per stream: warm-up + one partial iteration), one of a single 16-byte group (generic kernel between two
     fast ones), seven streams (a ragged share of the flattened work space), power requested on alternate chunks (both
-    template instantiations).  Baseband <= 1e-4 of the oracle's, power <= 0.01 dB."""
+    template instantiations).  /50 also feeds an aligned chunk with outputs but shorter than the tail, which the FFMA2
+    stream kernel fast::p25_ddc_fm_stream_kernel<u8> serves, and then a w50i chunk that starts from the tail it carried.
+    Baseband <= 1e-4 of the oracle's, power <= 0.01 dB."""
     fs = 240_000 * (dec // 5)
     S_ = 7
     total = sum(chunks)
