@@ -1,21 +1,9 @@
-"""Oracle demod chain (reference src/demod.rs:82-114) against independent scipy arithmetic."""
+"""Oracle demod chain (reference src/demod.rs:82-114) against the float64 restatement (oracle/demod_f64.py)."""
 import numpy as np
-import p25_spec as S
 import pytest
-from scipy import signal
+from oracle import demod_f64 as F
 from tools import p25tx as tx
 from util import check_against_truth
-
-
-def _scipy_chain(iq: np.ndarray, front: bool) -> np.ndarray:
-    x = iq.astype(np.complex128)
-    if front:
-        x = signal.lfilter(S.taps_front().astype(np.float64), 1.0, x)[9::10]
-    x = signal.lfilter(S.taps_decim().astype(np.float64), 1.0, x)[4::5]
-    x = signal.lfilter(S.taps_chan().astype(np.float64), 1.0, x)
-    prev = np.concatenate([[0], x[:-1]])
-    d = np.angle(x * np.conj(prev)) * float(S.FM_GAIN)
-    return signal.lfilter(np.ones(10) / 10, 1.0, d)
 
 
 @pytest.mark.parametrize("front", [False, True])
@@ -24,7 +12,7 @@ def test_cf32_chain_matches_scipy(oracle, front):
     st = tx.control_channel(1, 1)
     iq = tx.modulate_iq(st.dibits, fs, snr_db=30, cfo_hz=100.0, seed=1)[: fs // 20]
     got = oracle.DemodChain(oracle.FMT_CF32, front).feed(iq)
-    ref = _scipy_chain(iq, front)
+    ref = F.chain(iq, 50 if front else 5)[1]
     assert len(got) == len(iq) // (50 if front else 5)
     assert np.max(np.abs(got - ref[: len(got)])) < 2e-5
 
@@ -34,8 +22,7 @@ def test_u8_chain_and_lut(oracle):
     iq = tx.modulate_iq(st.dibits, 240_000, snr_db=30, seed=2)[:16384]
     u8 = tx.iq_to_u8(iq)
     got = oracle.DemodChain(oracle.FMT_U8, False).feed(u8)
-    lut = S.iq_lut()
-    ref = _scipy_chain(lut[u8[0::2]] + 1j * lut[u8[1::2]], False)
+    ref = F.chain(F.u8_to_c128(u8), 5)[1]
     assert len(got) == 3276                      # floor(16384 / 5), reference src/demod.rs:87
     assert np.max(np.abs(got - ref[:3276])) < 2e-5
 
