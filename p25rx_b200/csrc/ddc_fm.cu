@@ -41,6 +41,96 @@ __constant__ float c_iq_lut[256];
 static_assert(P25_TAPS_FRONT == 5 * P25_DECIM_FRONT, "front stage is a 10-phase x 5-tap polyphase matrix");
 static_assert(P25_TAPS_DECIM == 5 * P25_DECIM_NATIVE, "decimator is a 5-phase x 5-tap polyphase matrix");
 
+// Device primitives of the TMA-staged kernels (fast, w5, w5i, w50i): mbarriers, 1-D bulk copies, packed FP32, and the
+// packed atan2 of the warp kernels' discriminator.
+namespace prim {
+
+__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
+}
+__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
+    unsigned ok;
+    do {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+            : "=r"(ok)
+            : "r"(smem_u32(bar)), "r"(parity)
+            : "memory");
+    } while (!ok);
+}
+__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
+                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
+                 : "memory");
+}
+// acc += h * x on both components: one FFMA2
+__device__ __forceinline__ float2 cfma(float h, float2 x, float2 acc) {
+    unsigned long long r;
+    const float2 hh = make_float2(h, h);
+    asm("fma.rn.f32x2 %0, %1, %2, %3;"
+        : "=l"(r)
+        : "l"(*reinterpret_cast<const unsigned long long*>(&hh)), "l"(*reinterpret_cast<const unsigned long long*>(&x)),
+          "l"(*reinterpret_cast<const unsigned long long*>(&acc)));
+    return *reinterpret_cast<float2*>(&r);
+}
+__device__ __forceinline__ float2 add2(float2 a, float2 b) {
+    unsigned long long r;
+    asm("add.rn.f32x2 %0, %1, %2;"
+        : "=l"(r)
+        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)));
+    return *reinterpret_cast<float2*>(&r);
+}
+
+__device__ __forceinline__ float2 mul2(float2 a, float2 b) {
+    unsigned long long r;
+    asm("mul.rn.f32x2 %0, %1, %2;"
+        : "=l"(r)
+        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)));
+    return *reinterpret_cast<float2*>(&r);
+}
+__device__ __forceinline__ float2 fma2s(float2 a, float2 b, float c) {   // a * b + (c, c)
+    unsigned long long r;
+    const float2 cc = make_float2(c, c);
+    asm("fma.rn.f32x2 %0, %1, %2, %3;"
+        : "=l"(r)
+        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)),
+          "l"(*reinterpret_cast<const unsigned long long*>(&cc)));
+    return *reinterpret_cast<float2*>(&r);
+}
+// atan2 for the discriminator, two outputs at once: |error| <= 2e-7 rad (degree-7 minimax in t^2 on [0, 1], spec/gen_tables.py
+// style fit; CUDA's atan2f costs ~85 instructions with its special-case branches, this one ~22, branch-free).
+// atan2(0, 0) = 0 like std::atan2 on +0 arguments.  The polynomial and the three multiplies run packed (same arithmetic
+// per half).
+__device__ __forceinline__ float2 disc_atan2_pair(float2 y, float2 x) {
+    const float ax0 = fabsf(x.x), ay0 = fabsf(y.x), ax1 = fabsf(x.y), ay1 = fabsf(y.y);
+    const float mx0 = fmaxf(ax0, ay0), mn0 = fminf(ax0, ay0), mx1 = fmaxf(ax1, ay1), mn1 = fminf(ax1, ay1);
+    float rc0, rc1;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc0) : "f"(fmaxf(mx0, 1e-30f)));
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc1) : "f"(fmaxf(mx1, 1e-30f)));
+    const float2 t = mul2(make_float2(mn0, mn1), make_float2(rc0, rc1)), u = mul2(t, t);
+    float2 q = make_float2(-0.004295386839658022f, -0.004295386839658022f);
+    q = fma2s(q, u, 0.022737378254532814f);
+    q = fma2s(q, u, -0.057179518043994904f);
+    q = fma2s(q, u, 0.09735459089279175f);
+    q = fma2s(q, u, -0.13945257663726807f);
+    q = fma2s(q, u, 0.1995391547679901f);
+    q = fma2s(q, u, -0.3333050608634949f);
+    q = fma2s(q, u, 0.9999995231628418f);
+    const float2 r = mul2(q, t);
+    float r0 = r.x, r1 = r.y;
+    r0 = ay0 > ax0 ? 1.57079632679489662f - r0 : r0;
+    r1 = ay1 > ax1 ? 1.57079632679489662f - r1 : r1;
+    r0 = x.x < 0.f ? 3.14159265358979324f - r0 : r0;
+    r1 = x.y < 0.f ? 3.14159265358979324f - r1 : r1;
+    return make_float2(copysignf(r0, y.x), copysignf(r1, y.y));
+}
+
+}  // namespace prim
+
 template <bool FRONT>
 struct Cfg {
     static constexpr int MB = FRONT ? 64 : 256;         // 48 kHz outputs per block
@@ -338,6 +428,8 @@ __global__ void __launch_bounds__(Cfg<FRONT>::NT) p25_ddc_fm_kernel(const DdcPar
 // =====================================================================================================
 namespace fast {
 
+using namespace prim;
+
 constexpr int MB = 64;            // 48 kHz outputs per block
 constexpr int NT = 320;           // threads = front-stage columns per block
 constexpr int XN = MB * 50;       // input samples per block
@@ -375,46 +467,6 @@ struct __align__(128) Smem {
     float red[16];
     unsigned long long full[2];    // mbarriers
 };
-
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-    unsigned ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-// acc += h * x on both components: one FFMA2
-__device__ __forceinline__ float2 cfma(float h, float2 x, float2 acc) {
-    unsigned long long r;
-    const float2 hh = make_float2(h, h);
-    asm("fma.rn.f32x2 %0, %1, %2, %3;"
-        : "=l"(r)
-        : "l"(*reinterpret_cast<const unsigned long long*>(&hh)), "l"(*reinterpret_cast<const unsigned long long*>(&x)),
-          "l"(*reinterpret_cast<const unsigned long long*>(&acc)));
-    return *reinterpret_cast<float2*>(&r);
-}
-__device__ __forceinline__ float2 add2(float2 a, float2 b) {
-    unsigned long long r;
-    asm("add.rn.f32x2 %0, %1, %2;"
-        : "=l"(r)
-        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)));
-    return *reinterpret_cast<float2*>(&r);
-}
 
 // NS u8 samples starting at half-word ODD of wp[0] -> floats in byte units centred on 128 (PRMT builds the float
 // 2^23 + b in place, one packed add removes 2^23 + 128): 2 PRMT + 1 FADD2 per sample, no table, no I2F
@@ -675,79 +727,295 @@ __global__ void __maxnreg__(F<FMT>::MAXREG) p25_ddc_fm_stream_kernel(const DdcPa
   }
 }
 
-__device__ __forceinline__ float2 mul2(float2 a, float2 b) {
-    unsigned long long r;
-    asm("mul.rn.f32x2 %0, %1, %2;"
-        : "=l"(r)
-        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)));
-    return *reinterpret_cast<float2*>(&r);
-}
-__device__ __forceinline__ float2 fma2s(float2 a, float2 b, float c) {   // a * b + (c, c)
-    unsigned long long r;
-    const float2 cc = make_float2(c, c);
-    asm("fma.rn.f32x2 %0, %1, %2, %3;"
-        : "=l"(r)
-        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)),
-          "l"(*reinterpret_cast<const unsigned long long*>(&cc)));
-    return *reinterpret_cast<float2*>(&r);
-}
-// atan2 for the discriminator, two outputs at once: |error| <= 2e-7 rad (degree-7 minimax in t^2 on [0, 1], spec/gen_tables.py
-// style fit; CUDA's atan2f costs ~85 instructions with its special-case branches, this one ~22, branch-free).
-// atan2(0, 0) = 0 like std::atan2 on +0 arguments.  The polynomial and the three multiplies run packed (same arithmetic
-// per half).
-__device__ __forceinline__ float2 disc_atan2_pair(float2 y, float2 x) {
-    const float ax0 = fabsf(x.x), ay0 = fabsf(y.x), ax1 = fabsf(x.y), ay1 = fabsf(y.y);
-    const float mx0 = fmaxf(ax0, ay0), mn0 = fminf(ax0, ay0), mx1 = fmaxf(ax1, ay1), mn1 = fminf(ax1, ay1);
-    float rc0, rc1;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc0) : "f"(fmaxf(mx0, 1e-30f)));
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc1) : "f"(fmaxf(mx1, 1e-30f)));
-    const float2 t = mul2(make_float2(mn0, mn1), make_float2(rc0, rc1)), u = mul2(t, t);
-    float2 q = make_float2(-0.004295386839658022f, -0.004295386839658022f);
-    q = fma2s(q, u, 0.022737378254532814f);
-    q = fma2s(q, u, -0.057179518043994904f);
-    q = fma2s(q, u, 0.09735459089279175f);
-    q = fma2s(q, u, -0.13945257663726807f);
-    q = fma2s(q, u, 0.1995391547679901f);
-    q = fma2s(q, u, -0.3333050608634949f);
-    q = fma2s(q, u, 0.9999995231628418f);
-    const float2 r = mul2(q, t);
-    float r0 = r.x, r1 = r.y;
-    r0 = ay0 > ax0 ? 1.57079632679489662f - r0 : r0;
-    r1 = ay1 > ax1 ? 1.57079632679489662f - r1 : r1;
-    r0 = x.x < 0.f ? 3.14159265358979324f - r0 : r0;
-    r1 = x.y < 0.f ? 3.14159265358979324f - r1 : r1;
-    return make_float2(copysignf(r0, y.x), copysignf(r1, y.y));
-}
-
 }  // namespace fast
 
 
 // =====================================================================================================
-// /5 fast path for cf32 input (the reference's own chain at 240 kS/s; 16-byte aligned rows).  The FP32 pipe and the
-// issue slots, not HBM, are the limit of this shape (62 complex-by-real taps per 48 kHz output), and CTA barriers
-// between stages that keep only part of a CTA busy would stall both, so every warp is its own pipeline and the only
-// synchronisation is __syncwarp:
-//   * a warp walks a contiguous share of the flattened (stream, iteration) space, 124 outputs per iteration
-//     (31 lanes x 4; lane 31 only contributes its inputs' partial sums to lane 30), entering each stream or
-//     share with one discarded warm-up iteration, so the carried FIR histories live in per-warp shared memory;
-//   * lane 0 streams the raw 5.1 KB input slices with TMA bulk copies into a per-warp two-stage ring;
+// Warp-autonomous kernels (w5, w5i, w50i).  The FP32 pipe and the issue slots, not HBM, are the limit of the /5 shapes,
+// and CTA barriers between stages that keep only part of a CTA busy would stall both, so every warp is its own pipeline
+// and the only synchronisation is __syncwarp:
+//   * a warp walks a contiguous share of the flattened (stream, iteration) space, NOUT outputs per iteration, entering
+//     each stream or share with one discarded warm-up iteration, so the carried FIR histories live in per-warp shared
+//     memory;
+//   * lane 0 streams the raw input slices with TMA bulk copies into a per-warp ring of one or two stages;
+//   * the kernel's own decimator writes R outputs per lane as rows of the channel filter's window arrays;
+//   * the 48 kHz stages are common: the channel filter's R outputs stay in registers for the discriminator (the
+//     previous sample arrives by shuffle), only the discriminator rows go back to shared memory for the boxcar; stores
+//     are 16 bytes per lane.
+// A kernel supplies its slice geometry, its decimator and its shared-memory layout; this namespace does the rest.
+// =====================================================================================================
+namespace wk {
+
+using namespace prim;
+
+// bulk copy of the slice whose first input has logical index l0 (tail ++ chunk) into xs, completing on bar; 32-bit index
+// arithmetic, the slice that still overlaps the carried tail (first iterations of a chunk only) takes the two-copy path.
+// CLAMP: the part in front of the tail (l0 < 0: warm-up of a chunk's first piece) is skipped, the destination keeps its
+// offset.
+template <int ES, int AL, int XLEN, bool CLAMP>
+__device__ __forceinline__ void issue_slice(unsigned char* xs, unsigned long long* bar, int ht, int lend,
+                                            const unsigned char* tail, const unsigned char* chunk, int l0) {
+    const int la0 = l0 & ~(AL - 1);
+    const int la = CLAMP ? max(la0, 0) : la0;
+    const int lb = min(la0 + XLEN, lend);
+    unsigned char* const dst = xs + (la - la0) * ES;
+    if (la >= ht) {
+        const unsigned bytes = (unsigned)(lb - la) * ES;
+        mbar_expect_tx(bar, bytes);
+        tma_load_1d(dst, chunk + (size_t)(la - ht) * ES, bytes, bar);
+        return;
+    }
+    const int t1 = min(lb, ht);
+    const unsigned nt = (unsigned)(t1 - la), nc = (unsigned)(lb - t1);
+    mbar_expect_tx(bar, (nt + nc) * ES);
+    tma_load_1d(dst, tail + (size_t)la * ES, nt * ES, bar);
+    if (nc) tma_load_1d(dst + nt * ES, chunk, nc * ES, bar);
+}
+
+// Walks this warp's share [b0, b1) of the flattened (stream, iteration) space piece by piece: a piece is a run of stored
+// iterations of one stream preceded by one warm-up iteration (iteration it_first - 1; -1 = the inputs just before the
+// chunk, served by the carried tail) that only rebuilds the filter histories.  Lane 0 keeps NSTAGE slices in flight
+// through issue(stage, tail, chunk, l0), NSTAGE iterations ahead (possibly into the next piece); the slice of iteration
+// it lands in stage `use % NSTAGE` behind full[stage].  Per iteration dec(stage, it) consumes the slice and writes the
+// decimator rows, and back(nv, out, pw) runs the 48 kHz stages and stores nv outputs (none in the warm-up) from out.
+// At the end of a piece: power flush, raw-tail carry when the stream's chunk is complete, next stream.
+template <int NSTAGE, int WARPS, int R, int NOUT, int XNEW, int ES, typename Issue, typename Dec, typename Back>
+__device__ __forceinline__ void walk(const DdcParams& p, const unsigned its_per_stream, const int warp, const int lane,
+                                     const int l_base, unsigned long long* const full, const bool want_pw,
+                                     const float pw_scale, Issue issue, Dec dec, Back back) {
+    const unsigned gw = blockIdx.x * WARPS + warp, GW = gridDim.x * WARPS;
+    const unsigned long long total = (unsigned long long)p.n_streams * its_per_stream;
+    const unsigned long long b0 = total * gw / GW, b1 = total * (gw + 1ull) / GW;
+    if (b0 >= b1) return;
+    const int ips = (int)its_per_stream, n_out = (int)p.n_out;
+    const size_t row_bytes = (size_t)p.n * ES, tail_bytes = (size_t)p.ht * ES;
+    unsigned s = (unsigned)(b0 / its_per_stream);
+    int it_first = (int)(b0 % its_per_stream);
+    unsigned left = (unsigned)(b1 - b0);                   // stored iterations still to do
+    const unsigned char* chunk = (const unsigned char*)p.iq + s * row_bytes;
+    const unsigned char* tail = (const unsigned char*)p.tail_in + s * tail_bytes;
+    if (lane == 0) {                                        // warm-up (and first stored iteration) of the first piece
+#pragma unroll
+        for (int k = 0; k < NSTAGE; k++) issue(k, tail, chunk, l_base + XNEW * (it_first - 1 + k));
+    }
+    unsigned use = 0;
+
+    while (left) {
+      const int n_st = min(ips - it_first, (int)left);     // stored iterations of this piece
+      const int npiece = n_st + 1;
+      left -= (unsigned)n_st;
+      float* const out_lane = p.bb + (size_t)s * p.row_stride + P25CU_BB_HIST + R * lane;
+      float pw = 0.f;
+      for (int j = 0; j < npiece; j++, use++) {
+        const int it = it_first - 1 + j;
+        const int stage = use % NSTAGE;
+        const int nv = j ? min(n_out - NOUT * it, NOUT) : 0;     // j = 0 is the warm-up: nothing is stored
+        mbar_wait(&full[stage], (use / NSTAGE) & 1);
+        dec(stage, it);
+        __syncwarp();                                                                 // S1: slice consumed, rows visible
+        if (lane == 0) {
+            if (j + NSTAGE < npiece) issue(stage, tail, chunk, l_base + XNEW * (it + NSTAGE));
+            // else the next piece's iteration j + NSTAGE - 1 - npiece (its warm-up is -1); with one stage only the last
+            // iteration gets here and asks for that warm-up
+            else if (left) issue(stage, tail + tail_bytes, chunk + row_bytes, l_base + XNEW * (NSTAGE == 1 ? -1 : j + NSTAGE - 1 - npiece));
+        }
+        back(nv, out_lane + NOUT * it, pw);
+      }
+      // ---- end of the piece: flush power, carry the raw input tail when the stream's chunk is complete, next stream
+      if (want_pw) {
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) pw += __shfl_xor_sync(0xFFFFFFFFu, pw, o);
+          if (lane == 0) atomicAdd(p.power_sum + s, pw * pw_scale);
+      }
+      if (it_first + n_st == ips) {
+          const uint4* src = reinterpret_cast<const uint4*>(chunk + ((size_t)p.n - p.ht) * ES);
+          uint4* dst = reinterpret_cast<uint4*>((unsigned char*)p.tail_out + s * tail_bytes);
+          for (int i = lane; i < (int)(tail_bytes / 16); i += 32) dst[i] = src[i];
+      }
+      s++;
+      it_first = 0;
+      chunk += row_bytes;
+      tail += tail_bytes;
+    }
+}
+
+// The 48 kHz stages of one iteration, R outputs per lane on lanes [0, NL) (w5: lane 31 only feeds the decimator):
+//   * decimator outputs are rows of R samples split over R / 2 arrays of 16-byte pairs, ys rows apart:
+//     yd[q ys + i] = (y[R i + 2 q], y[R i + 2 q + 1]); rows 0 .. HROWS - 1 are the history, row HROWS + lane the lane's
+//     own outputs, so a lane's channel-filter window is the consecutive rows lane .. lane + HROWS;
+//   * discriminator outputs are rows of R split over R / 4 arrays of four, ds rows apart, DROWS history rows in front;
+//   * c_carry is the last channel-filter output of the previous iteration, pw the power of the stored outputs.
+template <int R, int NL, int HROWS, int DROWS>
+__device__ __forceinline__ void back_end(float4* const yd, const int ys, float4* const d, const int ds, const int lane,
+                                         const float dc, float2& c_carry, const bool want_pw, float& pw, const int nv,
+                                         float* const out) {
+    constexpr int NQ = R / 2, ND = R / 4;
+    static_assert(R % 4 == 0 && HROWS * R == P25_TAPS_CHAN - 1 && DROWS * R >= P25_BOXCAR - 1, "history rows");
+
+    // ---- channel-select FIR: outputs R lane + r, window = rows lane .. lane + HROWS (s = 40 + r - k), samples in order
+    float2 acc[R];
+#pragma unroll
+    for (int r = 0; r < R; r++) acc[r] = make_float2(dc, dc);
+#pragma unroll
+    for (int t = 0; t <= HROWS; t++) {
+#pragma unroll
+        for (int q = 0; q < NQ; q++) {
+            const float4 v = yd[q * ys + lane + t];
+            const float2 x[2] = {make_float2(v.x, v.y), make_float2(v.z, v.w)};
+#pragma unroll
+            for (int e = 0; e < 2; e++) {
+#pragma unroll
+                for (int r = 0; r < R; r++) {
+                    const int k = (P25_TAPS_CHAN - 1) + r - (R * t + 2 * q + e);
+                    if (k >= 0 && k < P25_TAPS_CHAN) acc[r] = cfma(c_taps_chan[k], x[e], acc[r]);
+                }
+            }
+        }
+    }
+    // ---- FM discriminator on the outputs in registers; the sample before comes from the lane below
+    float2 prev;
+    prev.x = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].x, 1);
+    prev.y = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].y, 1);
+    if (lane == 0) prev = c_carry;
+    c_carry.x = __shfl_sync(0xFFFFFFFFu, acc[R - 1].x, NL - 1);
+    c_carry.y = __shfl_sync(0xFFFFFFFFu, acc[R - 1].y, NL - 1);
+    float dd[R];
+#pragma unroll
+    for (int r = 0; r < R; r += 2) {
+        const float2 c0 = acc[r], c1 = acc[r + 1];
+        const float2 re = make_float2(c0.x * prev.x + c0.y * prev.y, c1.x * c0.x + c1.y * c0.y);
+        const float2 im = make_float2(c0.y * prev.x - c0.x * prev.y, c1.y * c0.x - c1.x * c0.y);
+        const float2 th = disc_atan2_pair(im, re);
+        dd[r] = th.x * P25_FM_GAIN;
+        dd[r + 1] = th.y * P25_FM_GAIN;
+        if (want_pw && R * lane + r < nv) pw += c0.x * c0.x + c0.y * c0.y;
+        if (want_pw && R * lane + r + 1 < nv) pw += c1.x * c1.x + c1.y * c1.y;
+        prev = c1;
+    }
+#pragma unroll
+    for (int h = 0; h < ND; h++) d[h * ds + DROWS + lane] = make_float4(dd[4 * h], dd[4 * h + 1], dd[4 * h + 2], dd[4 * h + 3]);
+    __syncwarp();                                                                     // S2
+
+    // ---- boxcar over d[o - 9 .. o], o = R lane + r: old[i] = d[R lane - 9 + i] from the DROWS rows below the lane's own
+    {
+        float old[P25_BOXCAR - 1];
+#pragma unroll
+        for (int i = 0; i < P25_BOXCAR - 1; i++) {
+            const int m = R * DROWS - (P25_BOXCAR - 1) + i;                           // sample m of rows lane ..
+            const float4 v = d[(m % R) / 4 * ds + lane + m / R];
+            old[i] = m % 4 == 0 ? v.x : m % 4 == 1 ? v.y : m % 4 == 2 ? v.z : v.w;
+        }
+        float sum[R];
+        float s0 = old[0] + old[1];
+#pragma unroll
+        for (int i = 2; i < P25_BOXCAR - 1; i++) s0 += old[i];
+        sum[0] = s0 + dd[0];
+#pragma unroll
+        for (int r = 1; r < R; r++) sum[r] = (sum[r - 1] - old[r - 1]) + dd[r];
+        const float kk = 1.0f / P25_BOXCAR;
+        const int o0 = R * lane;
+        if (o0 < nv) {
+            if (o0 + R - 1 < nv) {
+#pragma unroll
+                for (int h = 0; h < ND; h++)
+                    reinterpret_cast<float4*>(out)[h] = make_float4(sum[4 * h] * kk, sum[4 * h + 1] * kk, sum[4 * h + 2] * kk, sum[4 * h + 3] * kk);
+            } else {
+#pragma unroll
+                for (int r = 0; r < R; r++)
+                    if (o0 + r < nv) out[r] = sum[r] * kk;
+            }
+        }
+    }
+    // ---- roll the histories: rows NL .. of every array move to the front (HROWS decimator rows, DROWS discriminator rows)
+    if constexpr (R == 4) {                                 // a lane moves one row of both decimator arrays
+        float4 ra = make_float4(0.f, 0.f, 0.f, 0.f), rb = ra, rd = ra;
+        if (lane < HROWS) {
+            ra = yd[NL + lane];
+            rb = yd[ys + NL + lane];
+        }
+        if (lane < DROWS) rd = d[NL + lane];
+        __syncwarp();                                                                 // S3
+        if (lane < HROWS) {
+            yd[lane] = ra;
+            yd[ys + lane] = rb;
+        }
+        if (lane < DROWS) d[lane] = rd;
+    } else {                                                // R = 8: a lane moves one row of one array
+        float4 ry = make_float4(0.f, 0.f, 0.f, 0.f), rd = ry;
+        const int yq = lane / HROWS, yr = lane - HROWS * yq;
+        if (lane < NQ * HROWS) ry = yd[yq * ys + NL + yr];
+        if (lane < 2 * DROWS) rd = (lane & 1) ? d[ds + NL + (lane >> 1)] : d[NL + (lane >> 1)];
+        __syncwarp();                                                                 // S3
+        if (lane < NQ * HROWS) yd[yq * ys + yr] = ry;
+        if (lane < 2 * DROWS) {
+            if (lane & 1) d[ds + (lane >> 1)] = rd;
+            else d[lane >> 1] = rd;
+        }
+    }
+}
+
+}  // namespace wk
+
+
+// Integer tensor pipe helpers of the u8 kernels (w5i, w50i): mma.sync u8 x s8 with s32 accumulators whose start values
+// make them floats (see w5i below).
+namespace i8 {
+
+using namespace prim;
+
+__device__ __forceinline__ void imma(int (&d)[4], const unsigned (&a)[4], const uint2 b) {
+    asm("mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+        : "+r"(d[0]), "+r"(d[1]), "+r"(d[2]), "+r"(d[3])
+        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y));
+}
+// first k-step of a chain: the start value (one register for all four accumulators) is the C operand
+__device__ __forceinline__ void imma0(int (&d)[4], const unsigned (&a)[4], const uint2 b, const int (&c)[4]) {
+    asm("mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%11,%12,%13};"
+        : "=r"(d[0]), "=r"(d[1]), "=r"(d[2]), "=r"(d[3])
+        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y), "r"(c[0]), "r"(c[1]), "r"(c[2]), "r"(c[3]));
+}
+// 4-byte shared-memory load the compiler may not fuse with its neighbour (an 8-byte load would need four moves to put
+// the words into the fragment's register order)
+__device__ __forceinline__ unsigned lds32(unsigned addr) {
+    unsigned v;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
+    return v;
+}
+// the three start values as register quads that stay resident (opaque to the compiler, which otherwise rebuilds a
+// quad with four moves in front of every chain: 41 MOV per iteration)
+__device__ __forceinline__ void load_init(const int4* g_init, int (&init)[3][4]) {
+#pragma unroll
+    for (int l = 0; l < 3; l++) {
+        const int4 v = g_init[l];
+        init[l][0] = v.x; init[l][1] = v.y; init[l][2] = v.z; init[l][3] = v.w;
+    }
+}
+// accumulator pair h ((c0, c1) or (c2, c3)) of the three limbs -> y = 2^16 s2 + 2^8 s1 + s0 as one complex output:
+// one FADD2 per limb removes the start value 1.5 * 2^23, two FFMA2 combine the limbs with a single rounding
+__device__ __forceinline__ float2 limbs_to_float(const int (&acc)[3][4], const int h) {
+    const float2 unmagic = make_float2(-12582912.f, -12582912.f);
+    float2 f[3];
+#pragma unroll
+    for (int l = 0; l < 3; l++)
+        f[l] = add2(make_float2(__int_as_float(acc[l][2 * h]), __int_as_float(acc[l][2 * h + 1])), unmagic);
+    return cfma(65536.f, f[2], cfma(256.f, f[1], f[0]));
+}
+
+}  // namespace i8
+
+
+// =====================================================================================================
+// /5 fast path for cf32 input (the reference's own chain at 240 kS/s; 16-byte aligned rows), a warp kernel (above):
+//   * 124 outputs per iteration (31 lanes x 4; lane 31 only contributes its inputs' partial sums to lane 30);
+//   * the raw 5.1 KB input slices go into a two-stage ring;
 //   * decimator: a lane owns 20 consecutive inputs and forms its four outputs' own part plus the part it contributes
 //     to its left neighbour's last outputs, which neighbours exchange by warp shuffle (25 FFMA2 per output);
 //   * decimator outputs are kept as rows of four (two 16-byte halves in two arrays): a lane's 44-sample channel
-//     filter window is then 22 conflict-free LDS.128 of consecutive rows;
-//   * the channel filter's four outputs stay in registers for the discriminator (the previous sample arrives
-//     by shuffle), only the discriminator rows go back to shared memory for the boxcar; stores are 16 bytes
-//     per lane, 496 contiguous bytes per warp.
+//     filter window is then 22 conflict-free LDS.128 of consecutive rows; stores are 496 contiguous bytes per warp.
 // =====================================================================================================
 namespace w5 {
 
-using fast::cfma;
-using fast::mbar_init;
-using fast::mbar_expect_tx;
-using fast::mbar_wait;
-using fast::tma_load_1d;
-using fast::add2;
-using fast::disc_atan2_pair;
+using namespace prim;
 
 constexpr int R = 4;                        // outputs per lane
 constexpr int NOUT = 31 * R;                // 124 outputs per warp iteration
@@ -768,25 +1036,7 @@ struct __align__(128) WarpSm {
     float4 d4[DROWS + 32];
     unsigned long long full[2];
 };
-
-// bulk copy of the slice whose first input has logical index l0 (tail ++ chunk); 32-bit index arithmetic, the slice
-// that still overlaps the carried tail (first iterations of a chunk only) takes the two-copy path
-__device__ __forceinline__ void issue_slice(WarpSm& sm, int stage, int ht, int lend, const unsigned char* tail,
-                                            const unsigned char* chunk, int l0) {
-    const int la = l0 & ~(AL - 1);
-    const int lb = min(la + XLEN, lend);
-    if (la >= ht) {
-        const unsigned bytes = (unsigned)(lb - la) * ES;
-        mbar_expect_tx(&sm.full[stage], bytes);
-        tma_load_1d(&sm.xs[stage][0], chunk + (size_t)(la - ht) * ES, bytes, &sm.full[stage]);
-        return;
-    }
-    const int t1 = min(lb, ht);
-    const unsigned nt = (unsigned)(t1 - la), nc = (unsigned)(lb - t1);
-    mbar_expect_tx(&sm.full[stage], (nt + nc) * ES);
-    tma_load_1d(&sm.xs[stage][0], tail + (size_t)la * ES, nt * ES, &sm.full[stage]);
-    if (nc) tma_load_1d(&sm.xs[stage][nt * ES], chunk, nc * ES, &sm.full[stage]);
-}
+constexpr size_t SMEM = sizeof(WarpSm) * WARPS;         // dynamic shared memory per CTA
 
 __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_warp_kernel(const DdcParams p, const unsigned its_per_stream,
                                                                          const float dc, const float pw_scale) {
@@ -802,45 +1052,19 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_warp_kernel(const D
     for (int i = lane; i < DROWS + 32; i += 32) sm.d4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     __syncwarp();
 
-    // this warp's share [b0, b1) of the flattened (stream, iteration) space, walked piece by piece: a piece is a run of
-    // stored iterations of one stream preceded by one warm-up iteration (iteration it_first - 1; -1 = the inputs just
-    // before the chunk, served by the carried tail) that only rebuilds the filter histories
-    const unsigned gw = blockIdx.x * WARPS + warp, GW = gridDim.x * WARPS;
-    const unsigned long long total = (unsigned long long)p.n_streams * its_per_stream;
-    const unsigned long long b0 = total * gw / GW, b1 = total * (gw + 1ull) / GW;
-    if (b0 >= b1) return;
-    const int ips = (int)its_per_stream, ht = (int)p.ht, lend = (int)p.ht + (int)p.n, n_out = (int)p.n_out;
-    const size_t row_bytes = (size_t)p.n * ES, tail_bytes = (size_t)p.ht * ES;
+    const int ht = (int)p.ht, lend = (int)p.ht + (int)p.n;
     const int l_base = (int)(5 * (long long)p.m0 - (long long)p.a0) - 20 + ht;   // logical index of iteration 0's first input
     const bool want_pw = p.power_sum != nullptr;
-    unsigned s = (unsigned)(b0 / its_per_stream);
-    int it_first = (int)(b0 % its_per_stream);
-    unsigned left = (unsigned)(b1 - b0);                   // stored iterations still to do
-    const unsigned char* chunk = (const unsigned char*)p.iq + s * row_bytes;
-    const unsigned char* tail = (const unsigned char*)p.tail_in + s * tail_bytes;
-    if (lane == 0) {                                        // warm-up and first stored iteration of the first piece
-        issue_slice(sm, 0, ht, lend, tail, chunk, l_base + XNEW * (it_first - 1));
-        issue_slice(sm, 1, ht, lend, tail, chunk, l_base + XNEW * it_first);
-    }
     float2 c_carry = make_float2(0.f, 0.f);
-    unsigned use = 0;
-
-    while (left) {
-      const int n_st = min(ips - it_first, (int)left);     // stored iterations of this piece
-      const int npiece = n_st + 1;
-      left -= (unsigned)n_st;
-      float* const out_lane = p.bb + (size_t)s * p.row_stride + P25CU_BB_HIST + R * lane;
-      float pw = 0.f;
-      for (int j = 0; j < npiece; j++, use++) {
-        const int it = it_first - 1 + j;
-        const int stage = use & 1;
-        const int skew = (l_base + XNEW * it) & (AL - 1);
-        const int nv = j ? min(n_out - NOUT * it, NOUT) : 0;     // j = 0 is the warm-up: nothing is stored
-        mbar_wait(&sm.full[stage], (use >> 1) & 1);
-
-        // ---- /5 decimator: lane owns inputs [20 lane, 20 lane + 20)
-        float2 own[R];
-        {
+    wk::walk<2, WARPS, R, NOUT, XNEW, ES>(
+        p, its_per_stream, warp, lane, l_base, sm.full, want_pw, pw_scale,
+        [&](int stage, const unsigned char* tail, const unsigned char* chunk, int l0) {
+            wk::issue_slice<ES, AL, XLEN, false>(sm.xs[stage], &sm.full[stage], ht, lend, tail, chunk, l0);
+        },
+        [&](int stage, int it) {
+            // ---- /5 decimator: lane owns inputs [20 lane, 20 lane + 20)
+            const int skew = (l_base + XNEW * it) & (AL - 1);
+            float2 own[R];
             float2 x[5 * R];
             const int s0 = skew + 5 * R * lane;
             // 16-byte loads (two samples): half the wavefronts of LDS.64 at this 160-byte lane stride
@@ -880,106 +1104,12 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_warp_kernel(const D
                     own[r].y += __shfl_down_sync(0xFFFFFFFFu, lft[r].y, 1);
                 }
             }
-        }
-        sm.ydA[HROWS + lane] = make_float4(own[0].x, own[0].y, own[1].x, own[1].y);   // lane 31's row is never read
-        sm.ydB[HROWS + lane] = make_float4(own[2].x, own[2].y, own[3].x, own[3].y);
-        __syncwarp();                                                                 // S1: xs[stage] consumed, rows visible
-        if (lane == 0) {                                    // prefetch two iterations ahead (possibly into the next piece)
-            if (j + 2 < npiece) issue_slice(sm, stage, ht, lend, tail, chunk, l_base + XNEW * (it + 2));
-            else if (left) issue_slice(sm, stage, ht, lend, tail + tail_bytes, chunk + row_bytes, l_base + XNEW * (j + 1 - npiece));
-        }
-
-        // ---- channel-select FIR: outputs 4 lane + r, window = rows lane .. lane + 10 (44 samples, s = 40 + r - k)
-        float2 acc[R];
-#pragma unroll
-        for (int r = 0; r < R; r++) acc[r] = make_float2(dc, dc);
-#pragma unroll
-        for (int t = 0; t <= HROWS; t++) {
-            const float4 va = sm.ydA[lane + t], vb = sm.ydB[lane + t];
-            const float2 xs4[4] = {make_float2(va.x, va.y), make_float2(va.z, va.w), make_float2(vb.x, vb.y), make_float2(vb.z, vb.w)};
-#pragma unroll
-            for (int q = 0; q < 4; q++) {
-#pragma unroll
-                for (int r = 0; r < R; r++) {
-                    const int k = (P25_TAPS_CHAN - 1) + r - (4 * t + q);
-                    if (k >= 0 && k < P25_TAPS_CHAN) acc[r] = cfma(c_taps_chan[k], xs4[q], acc[r]);
-                }
-            }
-        }
-        // ---- FM discriminator on the four outputs in registers; the sample before comes from the lane below
-        float2 prev;
-        prev.x = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].x, 1);
-        prev.y = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].y, 1);
-        if (lane == 0) prev = c_carry;
-        c_carry.x = __shfl_sync(0xFFFFFFFFu, acc[R - 1].x, 30);
-        c_carry.y = __shfl_sync(0xFFFFFFFFu, acc[R - 1].y, 30);
-        float dd[R];
-        static_assert(R % 2 == 0, "the discriminator runs on output pairs");
-#pragma unroll
-        for (int r = 0; r < R; r += 2) {
-            const float2 c0 = acc[r], c1 = acc[r + 1];
-            const float2 re = make_float2(c0.x * prev.x + c0.y * prev.y, c1.x * c0.x + c1.y * c0.y);
-            const float2 im = make_float2(c0.y * prev.x - c0.x * prev.y, c1.y * c0.x - c1.x * c0.y);
-            const float2 th = disc_atan2_pair(im, re);
-            dd[r] = th.x * P25_FM_GAIN;
-            dd[r + 1] = th.y * P25_FM_GAIN;
-            if (want_pw && R * lane + r < nv) pw += c0.x * c0.x + c0.y * c0.y;
-            if (want_pw && R * lane + r + 1 < nv) pw += c1.x * c1.x + c1.y * c1.y;
-            prev = c1;
-        }
-        sm.d4[DROWS + lane] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-        __syncwarp();                                                                 // S2
-
-        // ---- boxcar over d[o - 9 .. o], o = 4 lane + r: rows lane .. lane + 2 hold d[4 lane - 12 .. 4 lane - 1]
-        {
-            const float a = sm.d4[lane].w;
-            const float4 b = sm.d4[lane + 1], c4 = sm.d4[lane + 2];
-            float s0 = a + b.x;
-            s0 += b.y; s0 += b.z; s0 += b.w; s0 += c4.x; s0 += c4.y; s0 += c4.z; s0 += c4.w; s0 += dd[0];
-            const float s1 = (s0 - a) + dd[1], s2 = (s1 - b.x) + dd[2], s3 = (s2 - b.y) + dd[3];
-            const float kk = 1.0f / P25_BOXCAR;
-            const int o0 = R * lane;
-            if (o0 < nv) {
-                float* out = out_lane + NOUT * it;
-                if (o0 + 3 < nv) *reinterpret_cast<float4*>(out) = make_float4(s0 * kk, s1 * kk, s2 * kk, s3 * kk);
-                else {
-                    out[0] = s0 * kk;
-                    if (o0 + 1 < nv) out[1] = s1 * kk;
-                    if (o0 + 2 < nv) out[2] = s2 * kk;
-                }
-            }
-        }
-        // ---- roll the histories: the last 10 decimator rows and 3 discriminator rows move to the front
-        float4 ra = make_float4(0.f, 0.f, 0.f, 0.f), rb = ra, rd = ra;
-        if (lane < HROWS) {
-            ra = sm.ydA[31 + lane];
-            rb = sm.ydB[31 + lane];
-        }
-        if (lane < DROWS) rd = sm.d4[31 + lane];
-        __syncwarp();                                                                 // S3
-        if (lane < HROWS) {
-            sm.ydA[lane] = ra;
-            sm.ydB[lane] = rb;
-        }
-        if (lane < DROWS) sm.d4[lane] = rd;
-
-      }
-      // ---- end of the piece: flush power, carry the raw input tail when the stream's chunk is complete, next stream
-      if (want_pw) {
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) pw += __shfl_xor_sync(0xFFFFFFFFu, pw, o);
-          if (lane == 0) atomicAdd(p.power_sum + s, pw * pw_scale);
-      }
-      if (it_first + n_st == ips) {
-          const uint4* src = reinterpret_cast<const uint4*>(chunk + ((size_t)p.n - p.ht) * ES);
-          uint4* dst = reinterpret_cast<uint4*>((unsigned char*)p.tail_out + s * tail_bytes);
-          for (int i = lane; i < (int)(tail_bytes / 16); i += 32) dst[i] = src[i];
-      }
-      s++;
-      it_first = 0;
-      chunk += row_bytes;
-      tail += tail_bytes;
-    }
+            sm.ydA[HROWS + lane] = make_float4(own[0].x, own[0].y, own[1].x, own[1].y);   // lane 31's row is never read
+            sm.ydB[HROWS + lane] = make_float4(own[2].x, own[2].y, own[3].x, own[3].y);
+        },
+        [&](int nv, float* out, float& pw) {
+            wk::back_end<R, 31, HROWS, DROWS>(sm.ydA, (int)(sm.ydB - sm.ydA), sm.d4, 0, lane, dc, c_carry, want_pw, pw, nv, out);
+        });
 }
 
 }  // namespace w5
@@ -1007,17 +1137,12 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_warp_kernel(const D
 //     pointers by 8 bytes, sk selects one of four B tables (a window holds sk + 60 <= 63 samples).
 //   * the k index is permuted so that a lane's eight words of a row are four 8-byte loads, and mma row g reads slice
 //     row 2 (g & 3) + (g >> 2): both halves of the warp then hit 32 different banks (row stride 20 words).
-// 128 outputs per iteration on all 32 lanes (no ghost lane); everything after the decimator is the warp kernel's code.
+// 128 outputs per iteration on all 32 lanes (no ghost lane); everything after the decimator is the common warp kernel code.
 // =====================================================================================================
 namespace w5i {
 
-using fast::mbar_init;
-using fast::mbar_expect_tx;
-using fast::mbar_wait;
-using fast::tma_load_1d;
-using fast::cfma;
-using fast::add2;
-using fast::disc_atan2_pair;
+using namespace prim;
+using namespace i8;
 
 constexpr int R = 8;                                    // outputs per lane
 constexpr int NOUT = 32 * R;                            // 256 outputs per warp iteration: two m-tiles of 16 rows x 8 outputs
@@ -1045,45 +1170,10 @@ struct __align__(128) WarpSm {
     float4 dA[DROWS + 32], dB[DROWS + 32];      // discriminator outputs: (d[8 i .. 8 i + 3]) | (d[8 i + 4 .. 8 i + 7])
     unsigned long long full[2];
 };
+constexpr size_t SMEM = sizeof(WarpSm) * WARPS + sizeof(uint2) * NB * 32;   // dynamic shared memory per CTA: + B table
 
 __device__ uint2 g_btab[4][NB][32];             // [sk][fragment][lane] = (b0, b1)
 __device__ int4 g_init[3];                      // accumulator start value of every limb, four times (one C operand quad)
-
-__device__ __forceinline__ void imma(int (&d)[4], const unsigned (&a)[4], const uint2 b) {
-    asm("mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+r"(d[0]), "+r"(d[1]), "+r"(d[2]), "+r"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y));
-}
-// first k-step of a chain: the start value (one register for all four accumulators) is the C operand
-__device__ __forceinline__ void imma0(int (&d)[4], const unsigned (&a)[4], const uint2 b, const int (&c)[4]) {
-    asm("mma.sync.aligned.m16n8k32.row.col.s32.u8.s8.s32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%11,%12,%13};"
-        : "=r"(d[0]), "=r"(d[1]), "=r"(d[2]), "=r"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b.x), "r"(b.y), "r"(c[0]), "r"(c[1]), "r"(c[2]), "r"(c[3]));
-}
-// 4-byte shared-memory load the compiler may not fuse with its neighbour (an 8-byte load would need four moves to put
-// the words into the fragment's register order)
-__device__ __forceinline__ unsigned lds32(unsigned addr) {
-    unsigned v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
-
-__device__ __forceinline__ void issue_slice(WarpSm& sm, int stage, int ht, int lend, const unsigned char* tail,
-                                            const unsigned char* chunk, int l0) {
-    const int la = l0 & ~(AL - 1);
-    const int lb = min(la + XLEN, lend);
-    if (la >= ht) {
-        const unsigned bytes = (unsigned)(lb - la) * ES;
-        mbar_expect_tx(&sm.full[stage], bytes);
-        tma_load_1d(&sm.xs[stage][0], chunk + (size_t)(la - ht) * ES, bytes, &sm.full[stage]);
-        return;
-    }
-    const int t1 = min(lb, ht);
-    const unsigned nt = (unsigned)(t1 - la), nc = (unsigned)(lb - t1);
-    mbar_expect_tx(&sm.full[stage], (nt + nc) * ES);
-    tma_load_1d(&sm.xs[stage][0], tail + (size_t)la * ES, nt * ES, &sm.full[stage]);
-    if (nc) tma_load_1d(&sm.xs[stage][nt * ES], chunk, nc * ES, &sm.full[stage]);
-}
 
 template <bool PW>                              // PW: accumulate the channel power (every fourth chunk in the reference's cadence)
 __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_imma_kernel(const DdcParams p, const unsigned its_per_stream,
@@ -1092,7 +1182,7 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_imma_kernel(const D
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     WarpSm& sm = reinterpret_cast<WarpSm*>(smem_raw)[warp];
     uint2* const btab = reinterpret_cast<uint2*>(smem_raw + sizeof(WarpSm) * WARPS);
-    const int ips = (int)its_per_stream, ht = (int)p.ht, lend = (int)p.ht + (int)p.n, n_out = (int)p.n_out;
+    const int ht = (int)p.ht, lend = (int)p.ht + (int)p.n;
     const int l_base = (int)(5 * (long long)p.m0 - (long long)p.a0) - 20 + ht;   // logical index of iteration 0's first input
     const int skew = l_base & (AL - 1);                     // the same for every iteration of every stream
     for (int e = threadIdx.x; e < NB * 32; e += 32 * WARPS) btab[e] = (&g_btab[skew & 3][0][0])[e];
@@ -1105,20 +1195,6 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_imma_kernel(const D
     for (int i = lane; i < DROWS + 32; i += 32) sm.dA[i] = sm.dB[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     __syncthreads();
 
-    const unsigned gw = blockIdx.x * WARPS + warp, GW = gridDim.x * WARPS;
-    const unsigned long long total = (unsigned long long)p.n_streams * its_per_stream;
-    const unsigned long long b0 = total * gw / GW, b1 = total * (gw + 1ull) / GW;
-    if (b0 >= b1) return;
-    const size_t row_bytes = (size_t)p.n * ES, tail_bytes = (size_t)p.ht * ES;
-    unsigned s = (unsigned)(b0 / its_per_stream);
-    int it_first = (int)(b0 % its_per_stream);
-    unsigned left = (unsigned)(b1 - b0);
-    const unsigned char* chunk = (const unsigned char*)p.iq + s * row_bytes;
-    const unsigned char* tail = (const unsigned char*)p.tail_in + s * tail_bytes;
-    if (lane == 0) {
-        issue_slice(sm, 0, ht, lend, tail, chunk, l_base + XNEW * (it_first - 1));
-        issue_slice(sm, 1, ht, lend, tail, chunk, l_base + XNEW * it_first);
-    }
     // fragment geometry: mma rows g and g + 8 of m-tile mt read slice rows 16 mt + drow and + 8; a lane's words of a
     // k-step are t and t + 4 of its eight (row stride 20 words: 32 different banks for any row permutation); the row
     // permutation puts the half-warps' stores on rows {0, 2, 4, 6} / {1, 3, 5, 7} (+ 8, + 16 ...) of two arrays each
@@ -1127,34 +1203,18 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_imma_kernel(const D
     const unsigned a_off = 80u * drow + 8u * (skew >> 2) + 4u * tig;
     const uint2* const bl = btab + lane;
     float2* const ydst = reinterpret_cast<float2*>(&sm.yd[tig >> 1][HROWS + drow]) + (tig & 1);
-    const float2 unmagic = make_float2(-12582912.f, -12582912.f);
-    float2 c_carry = make_float2(0.f, 0.f);
-    unsigned use = 0;
-    // the three start values as register quads that stay resident (opaque to the compiler, which otherwise rebuilds a
-    // quad with four moves in front of every chain: 41 MOV per iteration)
     int init[3][4];
-#pragma unroll
-    for (int l = 0; l < 3; l++) {
-        const int4 v = g_init[l];
-        init[l][0] = v.x; init[l][1] = v.y; init[l][2] = v.z; init[l][3] = v.w;
-    }
-
-    while (left) {
-      const int n_st = min(ips - it_first, (int)left);
-      const int npiece = n_st + 1;
-      left -= (unsigned)n_st;
-      float* const out_lane = p.bb + (size_t)s * p.row_stride + P25CU_BB_HIST + R * lane;
-      float pw = 0.f;
-      for (int j = 0; j < npiece; j++, use++) {
-        const int it = it_first - 1 + j;
-        const int stage = use & 1;
-        const int nv = j ? min(n_out - NOUT * it, NOUT) : 0;
-        mbar_wait(&sm.full[stage], (use >> 1) & 1);
-
-        // ---- /5 decimator on the integer tensor pipe: 36 IMMA, every B fragment loaded once for both m-tiles
-        {
+    load_init(g_init, init);
+    float2 c_carry = make_float2(0.f, 0.f);
+    wk::walk<2, WARPS, R, NOUT, XNEW, ES>(
+        p, its_per_stream, warp, lane, l_base, sm.full, PW, pw_scale,
+        [&](int stage, const unsigned char* tail, const unsigned char* chunk, int l0) {
+            wk::issue_slice<ES, AL, XLEN, false>(sm.xs[stage], &sm.full[stage], ht, lend, tail, chunk, l0);
+        },
+        [&](int stage, int) {
+            // ---- /5 decimator on the integer tensor pipe: 36 IMMA, every B fragment loaded once for both m-tiles
             int acc[2][2][3][4];
-            const unsigned xa = fast::smem_u32(sm.xs[stage]) + a_off;
+            const unsigned xa = smem_u32(sm.xs[stage]) + a_off;
 #pragma unroll
             for (int ks = 0; ks < 4; ks++) {
                 unsigned a[2][4];
@@ -1187,113 +1247,11 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) p25_ddc5_imma_kernel(const D
 #pragma unroll
                 for (int nt = 0; nt < 2; nt++)
 #pragma unroll
-                    for (int h = 0; h < 2; h++) {
-                        float2 f[3];
-#pragma unroll
-                        for (int l = 0; l < 3; l++)
-                            f[l] = add2(make_float2(__int_as_float(acc[mt][nt][l][2 * h]), __int_as_float(acc[mt][nt][l][2 * h + 1])), unmagic);
-                        ydst[2 * (2 * nt * YROWS + 16 * mt + 8 * h)] = cfma(65536.f, f[2], cfma(256.f, f[1], f[0]));
-                    }
-        }
-        __syncwarp();                                                                 // S1: xs[stage] consumed, rows visible
-        if (lane == 0) {
-            if (j + 2 < npiece) issue_slice(sm, stage, ht, lend, tail, chunk, l_base + XNEW * (it + 2));
-            else if (left) issue_slice(sm, stage, ht, lend, tail + tail_bytes, chunk + row_bytes, l_base + XNEW * (j + 1 - npiece));
-        }
-
-        // ---- channel-select FIR: outputs 8 lane + r, window = rows lane .. lane + 5 (48 samples, s = 40 + r - k)
-        float2 acc[R];
-#pragma unroll
-        for (int r = 0; r < R; r++) acc[r] = make_float2(dc, dc);
-#pragma unroll
-        for (int t = 0; t <= HROWS; t++) {
-#pragma unroll
-            for (int q = 0; q < 4; q++) {
-                const float4 v = sm.yd[q][lane + t];
-                const float2 x0 = make_float2(v.x, v.y), x1 = make_float2(v.z, v.w);
-#pragma unroll
-                for (int r = 0; r < R; r++) {
-                    const int k0 = (P25_TAPS_CHAN - 1) + r - (8 * t + 2 * q);
-                    if (k0 >= 0 && k0 < P25_TAPS_CHAN) acc[r] = cfma(c_taps_chan[k0], x0, acc[r]);
-                    if (k0 - 1 >= 0 && k0 - 1 < P25_TAPS_CHAN) acc[r] = cfma(c_taps_chan[k0 - 1], x1, acc[r]);
-                }
-            }
-        }
-        // ---- FM discriminator on the eight outputs in registers; the sample before comes from the lane below
-        float2 prev;
-        prev.x = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].x, 1);
-        prev.y = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].y, 1);
-        if (lane == 0) prev = c_carry;
-        c_carry.x = __shfl_sync(0xFFFFFFFFu, acc[R - 1].x, 31);
-        c_carry.y = __shfl_sync(0xFFFFFFFFu, acc[R - 1].y, 31);
-        float dd[R];
-#pragma unroll
-        for (int r = 0; r < R; r += 2) {
-            const float2 c0 = acc[r], c1 = acc[r + 1];
-            const float2 re = make_float2(c0.x * prev.x + c0.y * prev.y, c1.x * c0.x + c1.y * c0.y);
-            const float2 im = make_float2(c0.y * prev.x - c0.x * prev.y, c1.y * c0.x - c1.x * c0.y);
-            const float2 th = disc_atan2_pair(im, re);
-            dd[r] = th.x * P25_FM_GAIN;
-            dd[r + 1] = th.y * P25_FM_GAIN;
-            if (PW && R * lane + r < nv) pw += c0.x * c0.x + c0.y * c0.y;
-            if (PW && R * lane + r + 1 < nv) pw += c1.x * c1.x + c1.y * c1.y;
-            prev = c1;
-        }
-        sm.dA[DROWS + lane] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-        sm.dB[DROWS + lane] = make_float4(dd[4], dd[5], dd[6], dd[7]);
-        __syncwarp();                                                                 // S2
-
-        // ---- boxcar over d[o - 9 .. o], o = 8 lane + r: the row below holds d[8 lane - 8 .. 8 lane - 1]
-        {
-            const float4 o4 = sm.dB[lane], ha = sm.dA[lane + 1], hb = sm.dB[lane + 1];
-            const float old[R] = {o4.w, ha.x, ha.y, ha.z, ha.w, hb.x, hb.y, hb.z};
-            float sum[R];
-            float s0 = old[0] + old[1];
-            s0 += old[2]; s0 += old[3]; s0 += old[4]; s0 += old[5]; s0 += old[6]; s0 += old[7]; s0 += hb.w; s0 += dd[0];
-            sum[0] = s0;
-#pragma unroll
-            for (int r = 1; r < R; r++) sum[r] = (sum[r - 1] - old[r - 1]) + dd[r];
-            const float kk = 1.0f / P25_BOXCAR;
-            const int o0 = R * lane;
-            if (o0 < nv) {
-                float* out = out_lane + NOUT * it;
-                if (o0 + R - 1 < nv) {
-                    reinterpret_cast<float4*>(out)[0] = make_float4(sum[0] * kk, sum[1] * kk, sum[2] * kk, sum[3] * kk);
-                    reinterpret_cast<float4*>(out)[1] = make_float4(sum[4] * kk, sum[5] * kk, sum[6] * kk, sum[7] * kk);
-                } else {
-#pragma unroll
-                    for (int r = 0; r < R; r++)
-                        if (o0 + r < nv) out[r] = sum[r] * kk;
-                }
-            }
-        }
-        // ---- roll the histories: the last 5 decimator rows of the four arrays and 2 discriminator rows move to the front
-        float4 ry = make_float4(0.f, 0.f, 0.f, 0.f), rd = ry;
-        const int yq = lane / HROWS, yr = lane - HROWS * yq;
-        if (lane < 4 * HROWS) ry = sm.yd[yq][32 + yr];
-        if (lane < 2 * DROWS) rd = (lane & 1) ? sm.dB[32 + (lane >> 1)] : sm.dA[32 + (lane >> 1)];
-        __syncwarp();                                                                 // S3
-        if (lane < 4 * HROWS) sm.yd[yq][yr] = ry;
-        if (lane < 2 * DROWS) {
-            if (lane & 1) sm.dB[lane >> 1] = rd;
-            else sm.dA[lane >> 1] = rd;
-        }
-      }
-      if constexpr (PW) {
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) pw += __shfl_xor_sync(0xFFFFFFFFu, pw, o);
-          if (lane == 0) atomicAdd(p.power_sum + s, pw * pw_scale);
-      }
-      if (it_first + n_st == ips) {
-          const uint4* src = reinterpret_cast<const uint4*>(chunk + ((size_t)p.n - p.ht) * ES);
-          uint4* dst = reinterpret_cast<uint4*>((unsigned char*)p.tail_out + s * tail_bytes);
-          for (int i = lane; i < (int)(tail_bytes / 16); i += 32) dst[i] = src[i];
-      }
-      s++;
-      it_first = 0;
-      chunk += row_bytes;
-      tail += tail_bytes;
-    }
+                    for (int h = 0; h < 2; h++) ydst[2 * (2 * nt * YROWS + 16 * mt + 8 * h)] = limbs_to_float(acc[mt][nt], h);
+        },
+        [&](int nv, float* out, float& pw) {
+            wk::back_end<R, 32, HROWS, DROWS>(&sm.yd[0][0], YROWS, sm.dA, (int)(sm.dB - sm.dA), lane, dc, c_carry, PW, pw, nv, out);
+        });
 }
 
 // host side: the banded tap matrix in fragment order and the accumulator start values (p25_imma_tables.h, plain C++ so that
@@ -1319,23 +1277,15 @@ static const Tables& tables() {
 // y = 2^16 s2 + 2^8 s1 + s0 in one FADD2 per limb + two FFMA2.  28 k-steps x 3 limbs = 84 IMMA per 64 outputs; every B
 // fragment (21.5 KB table per CTA) is loaded once for the two m-tiles of a 128-output warp iteration.  The row stride of
 // 100 words puts the 32 lanes of every fragment load on 32 different banks; the four outputs of a row are one row of
-// the channel filter's window arrays.  The 48 kHz stages are the warp kernel's (4 outputs per lane).
+// the channel filter's window arrays.  The 48 kHz stages are the common warp kernel code (4 outputs per lane).
 // The warm-up iteration of a piece that starts a chunk reaches 6,640 samples back but only its last 50 outputs (2,740
 // samples, inside the 3,264-sample tail) have to be right: bytes in front of the tail are simply not copied, and whatever
 // lies in the buffer gives finite garbage in outputs nobody keeps.
 // =====================================================================================================
 namespace w50i {
 
-using fast::mbar_init;
-using fast::mbar_expect_tx;
-using fast::mbar_wait;
-using fast::tma_load_1d;
-using fast::cfma;
-using fast::add2;
-using fast::disc_atan2_pair;
-using w5i::imma;
-using w5i::imma0;
-using w5i::lds32;
+using namespace prim;
+using namespace i8;
 
 constexpr int D = 50;
 constexpr int G = P25_TAPS_FRONT + P25_DECIM_FRONT * (P25_TAPS_DECIM - 1);   // 290 combined taps
@@ -1363,30 +1313,10 @@ struct __align__(128) WarpSm {
     float4 d4[DROWS + 32];
     unsigned long long full;
 };
+constexpr size_t SMEM = sizeof(WarpSm) * WARPS + sizeof(uint2) * NB * 32;   // dynamic shared memory per CTA: + B table
 
 __device__ uint2 g_btab[2][NB][32];             // [skew & 1][fragment][lane]
 __device__ int4 g_init[3];
-
-// bulk copy of the slice whose first input has logical index l0 (tail ++ chunk); the part in front of the tail
-// (l0 < 0: warm-up of a chunk's first piece) is skipped, the destination keeps its offset
-__device__ __forceinline__ void issue_slice(WarpSm& sm, int ht, int lend, const unsigned char* tail,
-                                            const unsigned char* chunk, int l0) {
-    const int la0 = l0 & ~(AL - 1);
-    const int la = max(la0, 0);
-    const int lb = min(la0 + XLEN, lend);
-    unsigned char* dst = &sm.xs[(la - la0) * ES];
-    if (la >= ht) {
-        const unsigned bytes = (unsigned)(lb - la) * ES;
-        mbar_expect_tx(&sm.full, bytes);
-        tma_load_1d(dst, chunk + (size_t)(la - ht) * ES, bytes, &sm.full);
-        return;
-    }
-    const int t1 = min(lb, ht);
-    const unsigned nt = (unsigned)(t1 - la), nc = (unsigned)(lb - t1);
-    mbar_expect_tx(&sm.full, (nt + nc) * ES);
-    tma_load_1d(dst, tail + (size_t)la * ES, nt * ES, &sm.full);
-    if (nc) tma_load_1d(dst + nt * ES, chunk, nc * ES, &sm.full);
-}
 
 template <bool PW>
 __global__ void __launch_bounds__(32 * WARPS, 1) p25_ddc50_imma_kernel(const DdcParams p, const unsigned its_per_stream,
@@ -1395,7 +1325,7 @@ __global__ void __launch_bounds__(32 * WARPS, 1) p25_ddc50_imma_kernel(const Ddc
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     WarpSm& sm = reinterpret_cast<WarpSm*>(smem_raw)[warp];
     uint2* const btab = reinterpret_cast<uint2*>(smem_raw + sizeof(WarpSm) * WARPS);
-    const int ips = (int)its_per_stream, ht = (int)p.ht, lend = (int)p.ht + (int)p.n, n_out = (int)p.n_out;
+    const int ht = (int)p.ht, lend = (int)p.ht + (int)p.n;
     // logical index (tail ++ chunk) of the first input of iteration 0's window: output m uses 50 m + lbase + [-240, 49]
     const int l_base = (int)(D * (long long)p.m0 - (long long)p.a0) - (G - D) + ht;
     const int skew = l_base & (AL - 1);                     // the same for every iteration of every stream
@@ -1410,50 +1340,24 @@ __global__ void __launch_bounds__(32 * WARPS, 1) p25_ddc50_imma_kernel(const Ddc
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // the zeroed stage buffers are overwritten by bulk copies
     __syncthreads();
 
-    const unsigned gw = blockIdx.x * WARPS + warp, GW = gridDim.x * WARPS;
-    const unsigned long long total = (unsigned long long)p.n_streams * its_per_stream;
-    const unsigned long long b0 = total * gw / GW, b1 = total * (gw + 1ull) / GW;
-    if (b0 >= b1) return;
-    const size_t row_bytes = (size_t)p.n * ES, tail_bytes = (size_t)p.ht * ES;
-    unsigned s = (unsigned)(b0 / its_per_stream);
-    int it_first = (int)(b0 % its_per_stream);
-    unsigned left = (unsigned)(b1 - b0);
-    const unsigned char* chunk = (const unsigned char*)p.iq + s * row_bytes;
-    const unsigned char* tail = (const unsigned char*)p.tail_in + s * tail_bytes;
-    if (lane == 0) {
-        issue_slice(sm, ht, lend, tail, chunk, l_base + XNEW * (it_first - 1));
-    }
     // fragment geometry: mma rows g and g + 8 of m-tile mt read slice rows 16 mt + g and + 8 (400 bytes apart); the
     // lane's words of a k-step are t and t + 4 of its eight; (c0, c1) / (c2, c3) are output 4 row + t
     const int g = lane >> 2, tig = lane & 3;
     const unsigned a_off = 400u * g + 4u * (skew >> 1) + 4u * tig;
     const uint2* const bl = btab + lane;
     float2* const ydst = reinterpret_cast<float2*>(tig < 2 ? &sm.ydA[HROWS + g] : &sm.ydB[HROWS + g]) + (tig & 1);
-    const float2 unmagic = make_float2(-12582912.f, -12582912.f);
-    float2 c_carry = make_float2(0.f, 0.f);
-    unsigned use = 0;
     int init[3][4];
-#pragma unroll
-    for (int l = 0; l < 3; l++) {
-        const int4 v = g_init[l];
-        init[l][0] = v.x; init[l][1] = v.y; init[l][2] = v.z; init[l][3] = v.w;
-    }
-
-    while (left) {
-      const int n_st = min(ips - it_first, (int)left);
-      const int npiece = n_st + 1;
-      left -= (unsigned)n_st;
-      float* const out_lane = p.bb + (size_t)s * p.row_stride + P25CU_BB_HIST + R * lane;
-      float pw = 0.f;
-      for (int j = 0; j < npiece; j++, use++) {
-        const int it = it_first - 1 + j;
-        const int nv = j ? min(n_out - NOUT * it, NOUT) : 0;
-        mbar_wait(&sm.full, use & 1);
-
-        // ---- /50: 290-tap FIR on the raw bytes, 168 IMMA
-        {
+    load_init(g_init, init);
+    float2 c_carry = make_float2(0.f, 0.f);
+    wk::walk<1, WARPS, R, NOUT, XNEW, ES>(
+        p, its_per_stream, warp, lane, l_base, &sm.full, PW, pw_scale,
+        [&](int, const unsigned char* tail, const unsigned char* chunk, int l0) {
+            wk::issue_slice<ES, AL, XLEN, true>(sm.xs, &sm.full, ht, lend, tail, chunk, l0);
+        },
+        [&](int, int) {
+            // ---- /50: 290-tap FIR on the raw bytes, 168 IMMA
             int acc[2][3][4];
-            const unsigned xa = fast::smem_u32(sm.xs) + a_off;
+            const unsigned xa = smem_u32(sm.xs) + a_off;
 #pragma unroll
             for (int ks = 0; ks < KS; ks++) {
                 unsigned a[2][4];
@@ -1478,108 +1382,11 @@ __global__ void __launch_bounds__(32 * WARPS, 1) p25_ddc50_imma_kernel(const Ddc
 #pragma unroll
             for (int mt = 0; mt < 2; mt++)
 #pragma unroll
-                for (int h = 0; h < 2; h++) {
-                    float2 f[3];
-#pragma unroll
-                    for (int l = 0; l < 3; l++)
-                        f[l] = add2(make_float2(__int_as_float(acc[mt][l][2 * h]), __int_as_float(acc[mt][l][2 * h + 1])), unmagic);
-                    ydst[2 * (16 * mt + 8 * h)] = cfma(65536.f, f[2], cfma(256.f, f[1], f[0]));
-                }
-        }
-        __syncwarp();                                                                 // S1: xs consumed, rows visible
-        if (lane == 0) {
-            if (j + 1 < npiece) issue_slice(sm, ht, lend, tail, chunk, l_base + XNEW * (it + 1));
-            else if (left) issue_slice(sm, ht, lend, tail + tail_bytes, chunk + row_bytes, l_base - XNEW);
-        }
-
-        // ---- channel-select FIR: outputs 4 lane + r, window = rows lane .. lane + 10 (44 samples, s = 40 + r - k)
-        float2 acc[R];
-#pragma unroll
-        for (int r = 0; r < R; r++) acc[r] = make_float2(dc, dc);
-#pragma unroll
-        for (int t = 0; t <= HROWS; t++) {
-            const float4 va = sm.ydA[lane + t], vb = sm.ydB[lane + t];
-            const float2 xs4[4] = {make_float2(va.x, va.y), make_float2(va.z, va.w), make_float2(vb.x, vb.y), make_float2(vb.z, vb.w)};
-#pragma unroll
-            for (int q = 0; q < 4; q++) {
-#pragma unroll
-                for (int r = 0; r < R; r++) {
-                    const int k = (P25_TAPS_CHAN - 1) + r - (4 * t + q);
-                    if (k >= 0 && k < P25_TAPS_CHAN) acc[r] = cfma(c_taps_chan[k], xs4[q], acc[r]);
-                }
-            }
-        }
-        // ---- FM discriminator
-        float2 prev;
-        prev.x = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].x, 1);
-        prev.y = __shfl_up_sync(0xFFFFFFFFu, acc[R - 1].y, 1);
-        if (lane == 0) prev = c_carry;
-        c_carry.x = __shfl_sync(0xFFFFFFFFu, acc[R - 1].x, 31);
-        c_carry.y = __shfl_sync(0xFFFFFFFFu, acc[R - 1].y, 31);
-        float dd[R];
-#pragma unroll
-        for (int r = 0; r < R; r += 2) {
-            const float2 c0 = acc[r], c1 = acc[r + 1];
-            const float2 re = make_float2(c0.x * prev.x + c0.y * prev.y, c1.x * c0.x + c1.y * c0.y);
-            const float2 im = make_float2(c0.y * prev.x - c0.x * prev.y, c1.y * c0.x - c1.x * c0.y);
-            const float2 th = disc_atan2_pair(im, re);
-            dd[r] = th.x * P25_FM_GAIN;
-            dd[r + 1] = th.y * P25_FM_GAIN;
-            if (PW && R * lane + r < nv) pw += c0.x * c0.x + c0.y * c0.y;
-            if (PW && R * lane + r + 1 < nv) pw += c1.x * c1.x + c1.y * c1.y;
-            prev = c1;
-        }
-        sm.d4[DROWS + lane] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-        __syncwarp();                                                                 // S2
-
-        // ---- boxcar over d[o - 9 .. o], o = 4 lane + r: rows lane .. lane + 2 hold d[4 lane - 12 .. 4 lane - 1]
-        {
-            const float4 a4 = sm.d4[lane], b = sm.d4[lane + 1], c4 = sm.d4[lane + 2];
-            const float a = a4.w;
-            float s0 = a + b.x;
-            s0 += b.y; s0 += b.z; s0 += b.w; s0 += c4.x; s0 += c4.y; s0 += c4.z; s0 += c4.w; s0 += dd[0];
-            const float s1 = (s0 - a) + dd[1], s2 = (s1 - b.x) + dd[2], s3 = (s2 - b.y) + dd[3];
-            const float kk = 1.0f / P25_BOXCAR;
-            const int o0 = R * lane;
-            if (o0 < nv) {
-                float* out = out_lane + NOUT * it;
-                if (o0 + 3 < nv) *reinterpret_cast<float4*>(out) = make_float4(s0 * kk, s1 * kk, s2 * kk, s3 * kk);
-                else {
-                    out[0] = s0 * kk;
-                    if (o0 + 1 < nv) out[1] = s1 * kk;
-                    if (o0 + 2 < nv) out[2] = s2 * kk;
-                }
-            }
-        }
-        // ---- roll the histories: the last 10 decimator rows and 3 discriminator rows move to the front
-        float4 ra = make_float4(0.f, 0.f, 0.f, 0.f), rb = ra, rd = ra;
-        if (lane < HROWS) {
-            ra = sm.ydA[32 + lane];
-            rb = sm.ydB[32 + lane];
-        }
-        if (lane < DROWS) rd = sm.d4[32 + lane];
-        __syncwarp();                                                                 // S3
-        if (lane < HROWS) {
-            sm.ydA[lane] = ra;
-            sm.ydB[lane] = rb;
-        }
-        if (lane < DROWS) sm.d4[lane] = rd;
-      }
-      if constexpr (PW) {
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) pw += __shfl_xor_sync(0xFFFFFFFFu, pw, o);
-          if (lane == 0) atomicAdd(p.power_sum + s, pw * pw_scale);
-      }
-      if (it_first + n_st == ips) {
-          const uint4* src = reinterpret_cast<const uint4*>(chunk + ((size_t)p.n - p.ht) * ES);
-          uint4* dst = reinterpret_cast<uint4*>((unsigned char*)p.tail_out + s * tail_bytes);
-          for (int i = lane; i < (int)(tail_bytes / 16); i += 32) dst[i] = src[i];
-      }
-      s++;
-      it_first = 0;
-      chunk += row_bytes;
-      tail += tail_bytes;
-    }
+                for (int h = 0; h < 2; h++) ydst[2 * (16 * mt + 8 * h)] = limbs_to_float(acc[mt], h);
+        },
+        [&](int nv, float* out, float& pw) {
+            wk::back_end<R, 32, HROWS, DROWS>(sm.ydA, (int)(sm.ydB - sm.ydA), sm.d4, 0, lane, dc, c_carry, PW, pw, nv, out);
+        });
 }
 
 // host side: combined taps (double), limbs, banded matrix in fragment order, accumulator start values (p25_imma_tables.h)
@@ -1595,27 +1402,24 @@ static const Tables& tables() {
 
 unsigned p25cu_ddc_tail_len(int decimation) { return decimation == 50 ? Cfg<true>::HT : Cfg<false>::HT; }
 
+// the banded tap matrix and the accumulator start values (one C operand quad per limb) of an integer kernel
+template <typename T, typename B>
+static cudaError_t upload_imma(const T& t, const B& g_btab, const int4 (&g_init)[3]) {
+    if (!t.ok) return cudaErrorInvalidValue;
+    cudaError_t e = cudaMemcpyToSymbol(g_btab, t.b, sizeof(g_btab));
+    if (e != cudaSuccess) return e;
+    const int4 q[3] = {make_int4(t.init[0], t.init[0], t.init[0], t.init[0]), make_int4(t.init[1], t.init[1], t.init[1], t.init[1]),
+                       make_int4(t.init[2], t.init[2], t.init[2], t.init[2])};
+    return cudaMemcpyToSymbol(g_init, q, sizeof(q));
+}
+
 cudaError_t p25cu_ddc_upload_taps() {
     cudaError_t e;
     if ((e = cudaMemcpyToSymbol(c_taps_front, P25_TAPS_FRONT_H, sizeof(c_taps_front))) != cudaSuccess) return e;
     if ((e = cudaMemcpyToSymbol(c_taps_decim, P25_TAPS_DECIM_H, sizeof(c_taps_decim))) != cudaSuccess) return e;
     if ((e = cudaMemcpyToSymbol(c_taps_chan, P25_TAPS_CHAN_H, sizeof(c_taps_chan))) != cudaSuccess) return e;
-    {
-        const w5i::Tables& t = w5i::tables();
-        if (!t.ok) return cudaErrorInvalidValue;
-        if ((e = cudaMemcpyToSymbol(w5i::g_btab, t.b, sizeof(w5i::g_btab))) != cudaSuccess) return e;
-        const int4 q[3] = {make_int4(t.init[0], t.init[0], t.init[0], t.init[0]), make_int4(t.init[1], t.init[1], t.init[1], t.init[1]),
-                           make_int4(t.init[2], t.init[2], t.init[2], t.init[2])};
-        if ((e = cudaMemcpyToSymbol(w5i::g_init, q, sizeof(q))) != cudaSuccess) return e;
-    }
-    {
-        const w50i::Tables& t = w50i::tables();
-        if (!t.ok) return cudaErrorInvalidValue;
-        if ((e = cudaMemcpyToSymbol(w50i::g_btab, t.b, sizeof(w50i::g_btab))) != cudaSuccess) return e;
-        const int4 q[3] = {make_int4(t.init[0], t.init[0], t.init[0], t.init[0]), make_int4(t.init[1], t.init[1], t.init[1], t.init[1]),
-                           make_int4(t.init[2], t.init[2], t.init[2], t.init[2])};
-        if ((e = cudaMemcpyToSymbol(w50i::g_init, q, sizeof(q))) != cudaSuccess) return e;
-    }
+    if ((e = upload_imma(w5i::tables(), w5i::g_btab, w5i::g_init)) != cudaSuccess) return e;
+    if ((e = upload_imma(w50i::tables(), w50i::g_btab, w50i::g_init)) != cudaSuccess) return e;
     return cudaMemcpyToSymbol(c_iq_lut, P25_IQ_LUT, sizeof(c_iq_lut));
 }
 
@@ -1660,47 +1464,48 @@ static cudaError_t launch_fast(const DdcParams& p, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-static cudaError_t launch_w5(const DdcParams& p, cudaStream_t st) {
-    const size_t smem = sizeof(w5::WarpSm) * w5::WARPS;
-    const unsigned ips = (p.n_out + w5::NOUT - 1) / w5::NOUT;
+// Launch geometry of a warp kernel: iterations per stream, and a grid of at most grid_max CTAs that gives every warp at
+// least ~4 iterations (one warm-up each)
+struct WarpGrid {
+    unsigned ips, grid;
+};
+static WarpGrid warp_grid(const DdcParams& p, int nout, int warps, int grid_max) {
+    const unsigned ips = (p.n_out + nout - 1) / nout;
     const unsigned long long total = (unsigned long long)p.n_streams * ips;
-    unsigned long long want = (total + 3) / 4;                 // at least ~4 iterations per warp (one warm-up each)
-    want = (want + w5::WARPS - 1) / w5::WARPS;
-    const unsigned grid = want < (unsigned long long)p.plan->grid_w5 ? (unsigned)(want ? want : 1) : (unsigned)p.plan->grid_w5;
-    w5::p25_ddc5_warp_kernel<<<grid, 32 * w5::WARPS, smem, st>>>(p, ips, 0.f, 1.f);
+    unsigned long long want = (total + 3) / 4;
+    want = (want + warps - 1) / warps;
+    return {ips, want < (unsigned long long)grid_max ? (unsigned)(want ? want : 1) : (unsigned)grid_max};
+}
+
+// dc and power scale of an integer kernel: yd is in byte units x 2^scale_log2, so the half LSB of the u8 mapping enters
+// the channel filter at that scale
+struct ImmaScales {
+    float dc, pw_scale;
+};
+static ImmaScales imma_scales(double gain, int scale_log2) {
+    const double sc = (double)(1 << scale_log2);
+    return {(float)(0.5 * gain * tap_gain(P25_TAPS_CHAN_H, P25_TAPS_CHAN) * sc), (float)(1.0 / (127.5 * 127.5) / (sc * sc))};
+}
+
+static cudaError_t launch_w5(const DdcParams& p, cudaStream_t st) {
+    const WarpGrid g = warp_grid(p, w5::NOUT, w5::WARPS, p.plan->grid_w5);
+    w5::p25_ddc5_warp_kernel<<<g.grid, 32 * w5::WARPS, w5::SMEM, st>>>(p, g.ips, 0.f, 1.f);
     return cudaGetLastError();
 }
 
 static cudaError_t launch_w5i(const DdcParams& p, cudaStream_t st) {
-    const size_t smem = sizeof(w5i::WarpSm) * w5i::WARPS + sizeof(uint2) * w5i::NB * 32;
-    const unsigned ips = (p.n_out + w5i::NOUT - 1) / w5i::NOUT;
-    const unsigned long long total = (unsigned long long)p.n_streams * ips;
-    unsigned long long want = (total + 3) / 4;                 // at least ~4 iterations per warp (one warm-up each)
-    want = (want + w5i::WARPS - 1) / w5i::WARPS;
-    const unsigned grid = want < (unsigned long long)p.plan->grid_w5i ? (unsigned)(want ? want : 1) : (unsigned)p.plan->grid_w5i;
-    const w5i::Tables& t = w5i::tables();
-    // yd is in byte units x 2^25: the half LSB of the u8 mapping enters the channel filter at that scale
-    const double sc = (double)(1 << w5i::SCALE_LOG2);
-    const float dc = (float)(0.5 * t.gain * tap_gain(P25_TAPS_CHAN_H, P25_TAPS_CHAN) * sc);
-    const float pw_scale = (float)(1.0 / (127.5 * 127.5) / (sc * sc));
-    if (p.power_sum) w5i::p25_ddc5_imma_kernel<true><<<grid, 32 * w5i::WARPS, smem, st>>>(p, ips, dc, pw_scale);
-    else w5i::p25_ddc5_imma_kernel<false><<<grid, 32 * w5i::WARPS, smem, st>>>(p, ips, dc, pw_scale);
+    const WarpGrid g = warp_grid(p, w5i::NOUT, w5i::WARPS, p.plan->grid_w5i);
+    const ImmaScales k = imma_scales(w5i::tables().gain, w5i::SCALE_LOG2);
+    if (p.power_sum) w5i::p25_ddc5_imma_kernel<true><<<g.grid, 32 * w5i::WARPS, w5i::SMEM, st>>>(p, g.ips, k.dc, k.pw_scale);
+    else w5i::p25_ddc5_imma_kernel<false><<<g.grid, 32 * w5i::WARPS, w5i::SMEM, st>>>(p, g.ips, k.dc, k.pw_scale);
     return cudaGetLastError();
 }
 
 static cudaError_t launch_w50i(const DdcParams& p, cudaStream_t st) {
-    const size_t smem = sizeof(w50i::WarpSm) * w50i::WARPS + sizeof(uint2) * w50i::NB * 32;
-    const unsigned ips = (p.n_out + w50i::NOUT - 1) / w50i::NOUT;
-    const unsigned long long total = (unsigned long long)p.n_streams * ips;
-    unsigned long long want = (total + 3) / 4;                 // at least ~4 iterations per warp (one warm-up each)
-    want = (want + w50i::WARPS - 1) / w50i::WARPS;
-    const unsigned grid = want < (unsigned long long)p.plan->grid_w50i ? (unsigned)(want ? want : 1) : (unsigned)p.plan->grid_w50i;
-    const w50i::Tables& t = w50i::tables();
-    const double sc = (double)(1 << w50i::SCALE_LOG2);
-    const float dc = (float)(0.5 * t.gain * tap_gain(P25_TAPS_CHAN_H, P25_TAPS_CHAN) * sc);
-    const float pw_scale = (float)(1.0 / (127.5 * 127.5) / (sc * sc));
-    if (p.power_sum) w50i::p25_ddc50_imma_kernel<true><<<grid, 32 * w50i::WARPS, smem, st>>>(p, ips, dc, pw_scale);
-    else w50i::p25_ddc50_imma_kernel<false><<<grid, 32 * w50i::WARPS, smem, st>>>(p, ips, dc, pw_scale);
+    const WarpGrid g = warp_grid(p, w50i::NOUT, w50i::WARPS, p.plan->grid_w50i);
+    const ImmaScales k = imma_scales(w50i::tables().gain, w50i::SCALE_LOG2);
+    if (p.power_sum) w50i::p25_ddc50_imma_kernel<true><<<g.grid, 32 * w50i::WARPS, w50i::SMEM, st>>>(p, g.ips, k.dc, k.pw_scale);
+    else w50i::p25_ddc50_imma_kernel<false><<<g.grid, 32 * w50i::WARPS, w50i::SMEM, st>>>(p, g.ips, k.dc, k.pw_scale);
     return cudaGetLastError();
 }
 
@@ -1723,13 +1528,11 @@ cudaError_t p25cu_ddc_plan_device(P25DevPlan* plan) {
     constexpr int U8 = P25CU_FMT_U8_IQ, CF = P25CU_FMT_CF32_IQ;
     if ((e = plan_one(fast::p25_ddc_fm_stream_kernel<CF>, fast::NT, sizeof(fast::Smem<CF>), n_sm, &plan->grid_ddc50)) != cudaSuccess) return e;
     if ((e = plan_one(fast::p25_ddc_fm_stream_kernel<U8>, fast::NT, sizeof(fast::Smem<U8>), n_sm, &plan->grid_ddc50_u8)) != cudaSuccess) return e;
-    if ((e = plan_one(w5::p25_ddc5_warp_kernel, 32 * w5::WARPS, sizeof(w5::WarpSm) * w5::WARPS, n_sm, &plan->grid_w5)) != cudaSuccess) return e;
-    const size_t smem_w5i = sizeof(w5i::WarpSm) * w5i::WARPS + sizeof(uint2) * w5i::NB * 32;
-    if ((e = plan_one(w5i::p25_ddc5_imma_kernel<true>, 32 * w5i::WARPS, smem_w5i, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
-    if ((e = plan_one(w5i::p25_ddc5_imma_kernel<false>, 32 * w5i::WARPS, smem_w5i, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
-    const size_t smem_w50i = sizeof(w50i::WarpSm) * w50i::WARPS + sizeof(uint2) * w50i::NB * 32;
-    if ((e = plan_one(w50i::p25_ddc50_imma_kernel<true>, 32 * w50i::WARPS, smem_w50i, n_sm, &plan->grid_w50i)) != cudaSuccess) return e;
-    if ((e = plan_one(w50i::p25_ddc50_imma_kernel<false>, 32 * w50i::WARPS, smem_w50i, n_sm, &plan->grid_w50i)) != cudaSuccess) return e;
+    if ((e = plan_one(w5::p25_ddc5_warp_kernel, 32 * w5::WARPS, w5::SMEM, n_sm, &plan->grid_w5)) != cudaSuccess) return e;
+    if ((e = plan_one(w5i::p25_ddc5_imma_kernel<true>, 32 * w5i::WARPS, w5i::SMEM, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
+    if ((e = plan_one(w5i::p25_ddc5_imma_kernel<false>, 32 * w5i::WARPS, w5i::SMEM, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
+    if ((e = plan_one(w50i::p25_ddc50_imma_kernel<true>, 32 * w50i::WARPS, w50i::SMEM, n_sm, &plan->grid_w50i)) != cudaSuccess) return e;
+    if ((e = plan_one(w50i::p25_ddc50_imma_kernel<false>, 32 * w50i::WARPS, w50i::SMEM, n_sm, &plan->grid_w50i)) != cudaSuccess) return e;
     // the generic kernels' shared memory (27 - 72 KB) needs the opt-in as well
     if ((e = cudaFuncSetAttribute(p25_ddc_fm_kernel<true, U8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem<true>))) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(p25_ddc_fm_kernel<true, CF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem<true>))) != cudaSuccess) return e;
