@@ -11,16 +11,17 @@
 //
 // The whole chain is non-recursive, so every output is a pure function of a window of the logical
 // input (tail of the previous chunk ++ this chunk); the only carried state is that raw input tail,
-// kept in the stream's own sample format.  Five kernels share the arithmetic:
+// kept in the stream's own sample format.  Five kernels share the arithmetic; one of the last four takes every
+// chunk with outputs and 16-byte aligned rows, of any length, once a whole tail of the stream lies behind it (cf32 /50:
+// from the stream start on, given an even decimator phase), and the generic kernel takes the rest:
 //
 //   p25_ddc_fm_kernel<FRONT,FMT>      generic: any length and alignment, the first chunk of a stream
 //                                     (implicit zeros in front of it), odd chunks.  A CTA owns one
 //                                     (stream, segment), stages blocks with coalesced loads (u8 through
 //                                     a shared-memory copy of the table), runs the decimating stages
 //                                     input-stationary and the 48 kHz stages on power-of-two rings.
-//   fast::p25_ddc_fm_stream_kernel    /50: cf32 (the bench kernel), and u8 chunks shorter than the tail.
-//                                     TMA bulk copies into a two-stage ring, FFMA2 FIRs, persistent grid
-//                                     with a static + ticket work split.
+//   fast::p25_ddc_fm_stream_kernel    cf32 /50 (the bench kernel): TMA bulk copies into a two-stage ring,
+//                                     FFMA2 FIRs, persistent grid with a static + ticket work split.
 //   w5::p25_ddc5_warp_kernel          cf32 /5: warp-autonomous, every warp is its own pipeline, no CTA
 //                                     barriers.
 //   w5i::p25_ddc5_imma_kernel         u8 /5: the warp kernel with the /5 decimator as exact integer
@@ -436,28 +437,14 @@ constexpr int XN = MB * 50;       // input samples per block
 constexpr int ACOLS = 5 * MB;
 constexpr int HC = P25_TAPS_CHAN - 1;   // channel filter history (40)
 constexpr int HB = P25_BOXCAR - 1;      // boxcar history (9)
-
-// Per-format constants of the stream kernel.  cf32 blocks start on a 16-byte boundary by construction (even a0); u8
-// blocks (2 bytes per sample, 8 samples per 16 bytes) are staged from the enclosing aligned group and read with a skew.
-template <int FMT>
-struct F {
-    static constexpr bool U8 = FMT == P25CU_FMT_U8_IQ;
-    static constexpr int ES = U8 ? 2 : 8;                       // bytes per sample
-    static constexpr int AL = U8 ? 8 : 2;                       // samples per 16 bytes
-    static constexpr int XLEN = U8 ? XN + AL : XN;              // staged samples per block
-    static constexpr int XBYTES = (XLEN * ES + 127) / 128 * 128;
 #ifndef DDC50_MAXREG
 #define DDC50_MAXREG 56
 #endif
-#ifndef DDC50_U8_MAXREG
-#define DDC50_U8_MAXREG 48
-#endif
-    static constexpr int MAXREG = U8 ? DDC50_U8_MAXREG : DDC50_MAXREG;
-};
 
-template <int FMT>
+constexpr int ES = sizeof(float2);      // bytes per sample
+
 struct __align__(128) Smem {
-    unsigned char xs[2][F<FMT>::XBYTES];   // TMA destinations (raw samples of the stream's format)
+    unsigned char xs[2][XN * ES];  // TMA destinations (blocks start on a 16-byte boundary: even a0)
     float2 pa[4][ACOLS + 4];       // front partials q=1..4; slots 0..3 carry the previous block's last columns
     float2 ya[ACOLS];
     float2 pd[4][MB + 4];
@@ -467,26 +454,6 @@ struct __align__(128) Smem {
     float red[16];
     unsigned long long full[2];    // mbarriers
 };
-
-// NS u8 samples starting at half-word ODD of wp[0] -> floats in byte units centred on 128 (PRMT builds the float
-// 2^23 + b in place, one packed add removes 2^23 + 128): 2 PRMT + 1 FADD2 per sample, no table, no I2F
-template <int NS, bool ODD>
-__device__ __forceinline__ void load_u8n(const unsigned* __restrict__ wp, float2 (&x)[NS]) {
-    constexpr int NWORD = (NS + (ODD ? 1 : 0) + 1) / 2;
-    unsigned w[NWORD];
-#pragma unroll
-    for (int i = 0; i < NWORD; i++) w[i] = wp[i];
-    const float2 off = make_float2(-8388736.f, -8388736.f);   // -(2^23 + 128)
-#pragma unroll
-    for (int i = 0; i < NS; i++) {
-        const int hw = i + (ODD ? 1 : 0);
-        const unsigned word = w[hw >> 1];
-        // bytes {b, 0, 0, 0x4B}: the float 2^23 + b
-        const unsigned fi = __byte_perm(word, 0x4B000000u, (hw & 1) ? 0x7442u : 0x7440u);
-        const unsigned fq = __byte_perm(word, 0x4B000000u, (hw & 1) ? 0x7443u : 0x7441u);
-        x[i] = add2(make_float2(__uint_as_float(fi), __uint_as_float(fq)), off);
-    }
-}
 
 template <int D>
 __device__ __forceinline__ void partials(const float2 (&x)[D], const float* __restrict__ h, float2 (&P)[5]) {
@@ -499,15 +466,12 @@ __device__ __forceinline__ void partials(const float2 (&x)[D], const float* __re
     }
 }
 
-// issue the bulk copies of logical samples [l0, l0 + XN) (u8: from the enclosing 16-byte group on; clipped to the
-// data that exists) into xs[stage]
-template <int FMT>
-__device__ __forceinline__ void issue_block(Smem<FMT>& sm, int stage, const DdcParams& p, const unsigned char* tail,
+// issue the bulk copies of logical samples [l0, l0 + XN) (clipped to the data that exists) into xs[stage]
+__device__ __forceinline__ void issue_block(Smem& sm, int stage, const DdcParams& p, const unsigned char* tail,
                                             const unsigned char* chunk, long long l0) {
-    constexpr int ES = F<FMT>::ES;
     const long long ht = p.ht, lend = ht + (long long)p.n;
-    const long long la = l0 & ~(long long)(F<FMT>::AL - 1);
-    long long l1 = la + F<FMT>::XLEN;
+    const long long la = l0 & ~1LL;
+    long long l1 = la + XN;
     if (l1 > lend) l1 = lend;
     const long long t1 = l1 < ht ? l1 : ht;       // end of the part served by the tail
     const unsigned nt = la < t1 ? (unsigned)(t1 - la) : 0u;
@@ -531,16 +495,13 @@ __device__ __forceinline__ void issue_block(Smem<FMT>& sm, int stage, const DdcP
 #endif
 constexpr unsigned DYN_CH = DDC50_DYN_CH;
 
-// u8 input (declared extension: the reference's sample format at the 2.4 MS/s rate): samples stay in byte units
-// centred on 128 like in the /5 kernels below; `dc` restores the half-LSB offset after the (unit-DC-gain) filters,
-// `pw_scale` rescales the power.  For cf32 dc = 0 and pw_scale = 1.
-template <int FMT>
-__global__ void __maxnreg__(F<FMT>::MAXREG) p25_ddc_fm_stream_kernel(const DdcParams p, const unsigned blocks_per_stream,
-                                                                    const unsigned n_static, const unsigned n_tickets,
-                                                                    const unsigned ticket_base, const float dc, const float pw_scale) {
-    constexpr int ES = F<FMT>::ES;
+// dc = 0 and pw_scale = 1 (the channel filter's start value and the power scale) are launch arguments, not literals:
+// with literals ptxas schedules the kernel differently, and that schedule measured 1-2 % slower (NVIDIA B200, 1000 W).
+__global__ void __maxnreg__(DDC50_MAXREG) p25_ddc_fm_stream_kernel(const DdcParams p, const unsigned blocks_per_stream,
+                                                                  const unsigned n_static, const unsigned n_tickets,
+                                                                  const unsigned ticket_base, const float dc, const float pw_scale) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    Smem<FMT>& sm = *reinterpret_cast<Smem<FMT>*>(smem_raw);
+    Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
     __shared__ unsigned s_ticket;
     const int tid = threadIdx.x;
 
@@ -593,8 +554,8 @@ __global__ void __maxnreg__(F<FMT>::MAXREG) p25_ddc_fm_stream_kernel(const DdcPa
         const long long m_first = mb - MB;
         const int nblk = (int)((me - m_first + MB - 1) / MB);
         if (tid == 0) {
-            issue_block<FMT>(sm, use & 1, p, tail, chunk, 50 * m_first + lbase);
-            if (nblk > 1) issue_block<FMT>(sm, (use + 1) & 1, p, tail, chunk, 50 * (m_first + MB) + lbase);
+            issue_block(sm, use & 1, p, tail, chunk, 50 * m_first + lbase);
+            if (nblk > 1) issue_block(sm, (use + 1) & 1, p, tail, chunk, 50 * (m_first + MB) + lbase);
         }
         __syncthreads();
 
@@ -607,26 +568,19 @@ __global__ void __maxnreg__(F<FMT>::MAXREG) p25_ddc_fm_stream_kernel(const DdcPa
             float2 P[5];
             {
                 float2 x[10];
-                if constexpr (F<FMT>::U8) {
-                    const int s0 = (int)((50 * mi + lbase) & (F<FMT>::AL - 1)) + 10 * tid;   // skew inside the staged group
-                    const unsigned* wp = reinterpret_cast<const unsigned*>(sm.xs[stage]) + (s0 >> 1);
-                    if (s0 & 1) load_u8n<10, true>(wp, x);
-                    else load_u8n<10, false>(wp, x);
-                } else {
-                    const float4* src = reinterpret_cast<const float4*>(sm.xs[stage]) + 5 * tid;
+                const float4* src = reinterpret_cast<const float4*>(sm.xs[stage]) + 5 * tid;
 #pragma unroll
-                    for (int i = 0; i < 5; i++) {
-                        const float4 v = src[i];
-                        x[2 * i] = make_float2(v.x, v.y);
-                        x[2 * i + 1] = make_float2(v.z, v.w);
-                    }
+                for (int i = 0; i < 5; i++) {
+                    const float4 v = src[i];
+                    x[2 * i] = make_float2(v.x, v.y);
+                    x[2 * i + 1] = make_float2(v.z, v.w);
                 }
                 partials<10>(x, c_taps_front, P);
             }
 #pragma unroll
             for (int q = 1; q < 5; q++) sm.pa[q - 1][tid + 4] = P[q];
             __syncthreads();                                                  // B1: xs[stage] fully consumed
-            if (tid == 0 && blk + 2 < nblk) issue_block<FMT>(sm, stage, p, tail, chunk, 50 * (mi + 2 * MB) + lbase);
+            if (tid == 0 && blk + 2 < nblk) issue_block(sm, stage, p, tail, chunk, 50 * (mi + 2 * MB) + lbase);
             {
                 float2 a = P[0];
 #pragma unroll
@@ -717,10 +671,9 @@ __global__ void __maxnreg__(F<FMT>::MAXREG) p25_ddc_fm_stream_kernel(const DdcPa
             }
         }
         if (it1 == blocks_per_stream) {   // this piece ends the stream's chunk: write the tail for the next chunk
-            using ET = typename Elem<FMT>::T;
-            ET* tout = (ET*)p.tail_out + (size_t)s * p.ht;
+            float2* tout = (float2*)p.tail_out + (size_t)s * p.ht;
             for (int i = tid; i < (int)p.ht; i += NT)
-                tout[i] = load_logical_raw<FMT>(p, tail, chunk, (long long)p.n + i);
+                tout[i] = load_logical_raw<P25CU_FMT_CF32_IQ>(p, tail, chunk, (long long)p.n + i);
         }
         __syncthreads();
     }
@@ -828,9 +781,13 @@ __device__ __forceinline__ void walk(const DdcParams& p, const unsigned its_per_
           if (lane == 0) atomicAdd(p.power_sum + s, pw * pw_scale);
       }
       if (it_first + n_st == ips) {
-          const uint4* src = reinterpret_cast<const uint4*>(chunk + ((size_t)p.n - p.ht) * ES);
+          // the next chunk's tail is (tail ++ chunk)[n, n + ht): groups [0, nt) are the end of the old tail when the chunk
+          // is shorter than it, the rest the chunk's last bytes (aligned rows: whole 16-byte groups either way)
+          const int nt = row_bytes < tail_bytes ? (int)((tail_bytes - row_bytes) / 16) : 0;
+          const uint4* src = reinterpret_cast<const uint4*>(chunk + ((long long)p.n - (long long)p.ht) * ES);   // group i >= nt
           uint4* dst = reinterpret_cast<uint4*>((unsigned char*)p.tail_out + s * tail_bytes);
-          for (int i = lane; i < (int)(tail_bytes / 16); i += 32) dst[i] = src[i];
+          for (int i = lane; i < nt; i += 32) dst[i] = reinterpret_cast<const uint4*>(tail + row_bytes)[i];
+          for (int i = nt + lane; i < (int)(tail_bytes / 16); i += 32) dst[i] = src[i];
       }
       s++;
       it_first = 0;
@@ -1270,7 +1227,7 @@ static const Tables& tables() {
 // u8 at 2.4 MS/s (/50) with BOTH decimating stages on the integer tensor pipe (round 2).  The /10 front stage and the /5
 // decimator are linear and see nothing but bytes in front of them, so their cascade is ONE 290-tap FIR at 2.4 MS/s,
 // g[10 k + i] = hd[k] hf[i], decimating by 50 straight to the 48 kHz decimator output -- 290 exact integer MACs per
-// output and component instead of 250 + 21 FFMA2 (the stream kernel above is FP32-bound: 30 % of the FFMA2 peak at 28 %
+// output and component instead of 250 + 21 FFMA2 (on FFMA2 the u8 /50 chain is FP32-bound: 30 % of the FFMA2 peak at 28 %
 // of HBM).  Same scheme as w5i: raw bytes as the A operand (sixteen overlapping rows of the TMA-staged slice, 200 samples
 // = 400 bytes apart, four outputs per row = one n-tile), the taps as a banded s8 matrix in three balanced limbs of
 // t = round(g 2^28), accumulators started at the bit pattern of 1.5 * 2^23 - 128 * (limb sum) so that they are floats,
@@ -1423,18 +1380,26 @@ cudaError_t p25cu_ddc_upload_taps() {
     return cudaMemcpyToSymbol(c_iq_lut, P25_IQ_LUT, sizeof(c_iq_lut));
 }
 
+// The generic kernel: one CTA per (stream, segment).  A stream's outputs are split into segments of whole blocks, each
+// with its own warm-up block: about 16 CTAs per SM over all streams, but at least 8 blocks per segment.
 template <bool FRONT, int FMT>
-static cudaError_t launch(const DdcParams& p, cudaStream_t st) {
+static cudaError_t launch(const DdcParams& p_in, cudaStream_t st) {
     using C = Cfg<FRONT>;
-    auto kern = p25_ddc_fm_kernel<FRONT, FMT>;
+    DdcParams p = p_in;
+    const unsigned iters = (p.n_out + C::MB - 1) / C::MB;
+    unsigned want = (unsigned)((size_t)p.plan->n_sm * 16 / p.n_streams);
+    const unsigned cap = iters / 8;
+    if (want > cap) want = cap;
+    if (want < 1) want = 1;
+    const unsigned per = (iters + want - 1) / want;
+    p.seg_out = (per ? per : 1) * C::MB;
+    p.n_seg = p.n_out ? (p.n_out + p.seg_out - 1) / p.seg_out : 1;
     const size_t smem = sizeof(Smem<FRONT>);   // opted in per device by p25cu_ddc_plan_device
-    kern<<<p.n_streams * p.n_seg, C::NT, smem, st>>>(p);
+    p25_ddc_fm_kernel<FRONT, FMT><<<p.n_streams * p.n_seg, C::NT, smem, st>>>(p);
     return cudaGetLastError();
 }
 
-unsigned p25cu_ddc_block_out(int decimation) { return decimation == 50 ? Cfg<true>::MB : Cfg<false>::MB; }
-
-// DC gain of a tap set (double): u8 samples run through the fast kernels in byte units centred on 128,
+// DC gain of a tap set (double): u8 samples run through the integer kernels in byte units centred on 128,
 // x_true = (u - 128 + 0.5) / 127.5 (spec iq_lut), so the half LSB reappears after the filters as 0.5 * (product of gains)
 static double tap_gain(const float* h, int n) {
     double g = 0.0;
@@ -1442,11 +1407,8 @@ static double tap_gain(const float* h, int n) {
     return g;
 }
 
-template <int FMT>
 static cudaError_t launch_fast(const DdcParams& p, cudaStream_t st) {
-    constexpr bool U8 = FMT == P25CU_FMT_U8_IQ;
-    const size_t smem = sizeof(fast::Smem<FMT>);
-    const int grid_max = U8 ? p.plan->grid_ddc50_u8 : p.plan->grid_ddc50;
+    const int grid_max = p.plan->grid_ddc50;
     const unsigned bps = (p.n_out + fast::MB - 1) / fast::MB;
     const unsigned long long total = (unsigned long long)p.n_streams * bps;
     const unsigned grid = total < (unsigned long long)grid_max ? (unsigned)total : (unsigned)grid_max;
@@ -1455,11 +1417,7 @@ static cudaError_t launch_fast(const DdcParams& p, cudaStream_t st) {
     const unsigned n_static = (unsigned)(total / grid * DDC50_STATIC_NUM / DDC50_STATIC_DEN);
     const unsigned long long dyn = total - (unsigned long long)n_static * grid;
     const unsigned n_tickets = (unsigned)((dyn + fast::DYN_CH - 1) / fast::DYN_CH);
-    const float dc = U8 ? (float)(0.5 * tap_gain(P25_TAPS_FRONT_H, P25_TAPS_FRONT) * tap_gain(P25_TAPS_DECIM_H, P25_TAPS_DECIM) *
-                                  tap_gain(P25_TAPS_CHAN_H, P25_TAPS_CHAN))
-                        : 0.f;
-    const float pw_scale = U8 ? (float)(1.0 / (127.5 * 127.5)) : 1.f;
-    fast::p25_ddc_fm_stream_kernel<FMT><<<grid, fast::NT, smem, st>>>(p, bps, n_static, n_tickets, *p.ticket_base, dc, pw_scale);
+    fast::p25_ddc_fm_stream_kernel<<<grid, fast::NT, sizeof(fast::Smem), st>>>(p, bps, n_static, n_tickets, *p.ticket_base, 0.f, 1.f);
     *p.ticket_base += n_tickets + grid;
     return cudaGetLastError();
 }
@@ -1526,8 +1484,7 @@ cudaError_t p25cu_ddc_plan_device(P25DevPlan* plan) {
     cudaError_t e;
     const int n_sm = plan->n_sm;
     constexpr int U8 = P25CU_FMT_U8_IQ, CF = P25CU_FMT_CF32_IQ;
-    if ((e = plan_one(fast::p25_ddc_fm_stream_kernel<CF>, fast::NT, sizeof(fast::Smem<CF>), n_sm, &plan->grid_ddc50)) != cudaSuccess) return e;
-    if ((e = plan_one(fast::p25_ddc_fm_stream_kernel<U8>, fast::NT, sizeof(fast::Smem<U8>), n_sm, &plan->grid_ddc50_u8)) != cudaSuccess) return e;
+    if ((e = plan_one(fast::p25_ddc_fm_stream_kernel, fast::NT, sizeof(fast::Smem), n_sm, &plan->grid_ddc50)) != cudaSuccess) return e;
     if ((e = plan_one(w5::p25_ddc5_warp_kernel, 32 * w5::WARPS, w5::SMEM, n_sm, &plan->grid_w5)) != cudaSuccess) return e;
     if ((e = plan_one(w5i::p25_ddc5_imma_kernel<true>, 32 * w5i::WARPS, w5i::SMEM, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
     if ((e = plan_one(w5i::p25_ddc5_imma_kernel<false>, 32 * w5i::WARPS, w5i::SMEM, n_sm, &plan->grid_w5i)) != cudaSuccess) return e;
@@ -1542,20 +1499,15 @@ cudaError_t p25cu_ddc_plan_device(P25DevPlan* plan) {
 
 cudaError_t p25cu_launch_ddc(const DdcParams& p, int format, int decimation, cudaStream_t st) {
     if (p.n_out == 0 && p.n == 0) return cudaSuccess;
-    // /5 fast paths: aligned rows, the whole history inside the stream (no implicit zeros), chunk at least one tail long
-    if (decimation == 5 && p.aligned16 && p.n_out > 0 && p.a0 >= p.ht && p.n >= p.ht && p.ht == (unsigned)Cfg<false>::HT)
+    // warp kernels: aligned rows of any length, any decimator phase, and the whole history inside the stream (no implicit
+    // zeros: no u8 byte encodes them)
+    const bool warp = p.aligned16 && p.n_out > 0 && p.a0 >= p.ht;
+    if (decimation == 5 && warp && p.ht == (unsigned)Cfg<false>::HT)
         return format == P25CU_FMT_CF32_IQ ? launch_w5(p, st) : launch_w5i(p, st);
     if (decimation == 50 && format == P25CU_FMT_CF32_IQ && p.aligned16 && (p.a0 & 1ull) == 0 && p.n_out > 0 &&
         p.ht == (unsigned)Cfg<true>::HT)
-        return launch_fast<P25CU_FMT_CF32_IQ>(p, st);
-    // u8 at 2.4 MS/s: any decimator phase (blocks are staged from their enclosing 16-byte group); like the /5 fast paths the
-    // whole history must lie inside the stream (no byte encodes the zeros in front of a stream start)
-    if (decimation == 50 && format == P25CU_FMT_U8_IQ && p.aligned16 && p.n_out > 0 && p.a0 >= p.ht && p.ht == (unsigned)Cfg<true>::HT) {
-        // both decimating stages on the integer tensor pipe; it carries the tail from the chunk itself, so a chunk
-        // shorter than the tail takes the FFMA2 stream kernel
-        if (p.n >= p.ht) return launch_w50i(p, st);
-        return launch_fast<P25CU_FMT_U8_IQ>(p, st);
-    }
+        return launch_fast(p, st);
+    if (decimation == 50 && format == P25CU_FMT_U8_IQ && warp && p.ht == (unsigned)Cfg<true>::HT) return launch_w50i(p, st);
     if (decimation == 50)
         return format == P25CU_FMT_CF32_IQ ? launch<true, P25CU_FMT_CF32_IQ>(p, st) : launch<true, P25CU_FMT_U8_IQ>(p, st);
     return format == P25CU_FMT_CF32_IQ ? launch<false, P25CU_FMT_CF32_IQ>(p, st) : launch<false, P25CU_FMT_U8_IQ>(p, st);

@@ -14,7 +14,6 @@
 
 #include "p25cu_internal.cuh"
 
-unsigned p25cu_ddc_block_out(int decimation);
 cudaError_t p25cu_walk_upload_consts();
 // wideband channelizer (pfb.cu)
 unsigned p25cu_pfb_tail_len();
@@ -338,17 +337,6 @@ extern "C" int p25cu_demod(p25cu_ctx* ctx, const void* iq, size_t n, int iq_on_d
     p.ticket_base = &ctx->ticket_base;
     // every stream's row must start 16-byte aligned: 2 cf32 or 8 u8 samples per 16-byte load
     p.aligned16 = ((n % (ctx->cfg.format == P25CU_FMT_U8_IQ ? 8 : 2)) == 0) && (((uintptr_t)d_in & 15) == 0);
-    {
-        const unsigned mb = p25cu_ddc_block_out(D);
-        const unsigned iters = (p.n_out + mb - 1) / mb;
-        unsigned want = (unsigned)((size_t)ctx->n_sm * 16 / S);
-        unsigned cap = iters / 8;
-        if (want > cap) want = cap;
-        if (want < 1) want = 1;
-        const unsigned per = (iters + want - 1) / want;
-        p.seg_out = (per ? per : 1) * mb;
-        p.n_seg = p.n_out ? (p.n_out + p.seg_out - 1) / p.seg_out : 1;
-    }
     if (power_dbm) CK(cudaMemsetAsync(ctx->d_power, 0, S * sizeof(float), ctx->stream));
     const bool timed = ctx->timing && n && ctx->n_timed < 128;
     if (timed) CK(cudaEventRecord(ctx->tev[2 * ctx->n_timed], ctx->stream));

@@ -82,8 +82,7 @@ __host__ __device__ inline unsigned p25cu_packed_words(unsigned len) { return 3u
 struct P25DevPlan {
     int device;
     int n_sm;
-    int grid_ddc50;               // persistent grid of fast::p25_ddc_fm_stream_kernel
-    int grid_ddc50_u8;            // ... of its u8 instantiation
+    int grid_ddc50;               // persistent grid of fast::p25_ddc_fm_stream_kernel (cf32 /50)
     int grid_w5;                  // w5::p25_ddc5_warp_kernel (cf32 /5)
     int grid_w50i;                // w50i::p25_ddc50_imma_kernel (u8 /50, both decimating stages on the integer tensor pipe)
     int grid_w5i;                 // w5i::p25_ddc5_imma_kernel (u8, decimator on the integer tensor pipe)
@@ -103,8 +102,8 @@ struct DdcParams {
     unsigned n;                   // input samples per stream in this chunk
     unsigned n_out;               // outputs per stream in this chunk
     unsigned n_streams;
-    unsigned seg_out;             // outputs per segment (multiple of the per-iteration block)
-    unsigned n_seg;               // segments per stream
+    unsigned seg_out;             // generic kernel: outputs per segment (whole blocks), set by its launcher
+    unsigned n_seg;               // generic kernel: segments per stream, set by its launcher
     unsigned ht;                  // tail length in samples
     int aligned16;                // every chunk row starts 16-byte aligned and holds whole 16-byte groups
     unsigned* work_counter;       // device ticket counter of the /50 kernel's dynamic work split (monotonic)

@@ -56,29 +56,30 @@ SWEEP_ROWS = [(0.5, 0.0, 25, False), (0.9, 300.0, 25, False), (0.03, -200.0, 30,
               (0.3, 0.0, 25, True), (0.7, -450.0, 25, False), (0.25, 80.0, 20, True), (0.85, 600.0, 20, False)]
 
 # Chunk plans: (input samples, power requested, route).  Routes follow p25cu_launch_ddc (ddc_fm.cu):
-#   /5:  aligned rows (even cf32 / multiple-of-8 u8 length), a0 >= 1312 and n >= 1312 -> w5 (cf32) / w5i (u8);
-#        anything else (the first chunk, odd lengths) -> generic p25_ddc_fm_kernel<false, FMT>
-#   /50 cf32: aligned rows and an even a0 -> fast::p25_ddc_fm_stream_kernel<cf32>, else generic <true, cf32>
-#   /50 u8: aligned rows and a0 >= 3264 -> w50i when n >= 3264, fast::p25_ddc_fm_stream_kernel<u8> when shorter;
-#        else generic <true, u8>
-# The generic kernel splits a stream into segments when a chunk has >= 16 blocks of outputs (p25cu_api.cu): the
-# first chunk of each plan is one segment, the second several.  fast::p25_ddc_fm_stream_kernel<u8> only takes chunks
-# shorter than the tail (65 outputs): six of them in a row give the mutant checks enough of its outputs.
+#   /5:  chunks with outputs, aligned rows (even cf32 / multiple-of-8 u8 length) and a0 >= 1312, of any length
+#        -> w5 (cf32) / w5i (u8); anything else (the first chunk, odd lengths) -> generic p25_ddc_fm_kernel<false, FMT>
+#   /50 cf32: aligned rows and an even a0 -> fast::p25_ddc_fm_stream_kernel, else generic <true, cf32>
+#   /50 u8: aligned rows and a0 >= 3264, of any length -> w50i; else generic <true, u8>
+# The generic kernel splits a stream into segments when a chunk has >= 16 blocks of outputs (ddc_fm.cu): the first
+# chunk of each plan is one segment, the second several.  The warp kernels also take chunks shorter than the carried
+# tail (1,312 / 3,264 samples), down to one or two outputs, and carry the tail of such a chunk from the old tail and
+# the chunk; the chunk after each one starts from that tail.
 PLANS = {
-    ("cf32", 5): [(777, True, "generic"), (30001, True, "generic_seg"), (16384, True, "w5"), (1312, False, "w5")],
+    ("cf32", 5): [(777, True, "generic"), (30001, True, "generic_seg"), (16384, True, "w5"), (1312, False, "w5"),
+                  (1304, True, "w5"), (6, False, "w5"), (650, True, "w5")],
     ("u8", 5): [(777, True, "generic"), (30001, False, "generic_seg"), (16384, True, "w5i_pw"), (16384, False, "w5i"),
-                (1312, True, "w5i_pw")],
+                (1312, True, "w5i_pw"), (1304, False, "w5i"), (8, True, "w5i_pw"), (648, False, "w5i")],
     ("cf32", 50): [(47999, True, "generic"), (100001, False, "generic_seg"), (40000, True, "fast"), (40000, False, "fast")],
     ("u8", 50): [(47999, True, "generic"), (100001, True, "generic_seg"), (40000, True, "w50i_pw"), (40000, False, "w50i")] +
-                [(3256, i % 2 == 0, "fast") for i in range(6)] + [(3264, True, "w50i_pw")],
+                [(3256, i % 2 == 0, "w50i_pw" if i % 2 == 0 else "w50i") for i in range(6)] + [(3264, True, "w50i_pw")],
 }
 
 # route -> the kernel the profiler must see
 KERNELS = {("cf32", 5, "generic"): "p25_ddc_fm_kernel<false,1>", ("u8", 5, "generic"): "p25_ddc_fm_kernel<false,0>",
            ("cf32", 50, "generic"): "p25_ddc_fm_kernel<true,1>", ("u8", 50, "generic"): "p25_ddc_fm_kernel<true,0>",
            ("cf32", 5, "w5"): "w5::p25_ddc5_warp_kernel", ("u8", 5, "w5i_pw"): "w5i::p25_ddc5_imma_kernel<true>",
-           ("u8", 5, "w5i"): "w5i::p25_ddc5_imma_kernel<false>", ("cf32", 50, "fast"): "fast::p25_ddc_fm_stream_kernel<1>",
-           ("u8", 50, "fast"): "fast::p25_ddc_fm_stream_kernel<0>", ("u8", 50, "w50i_pw"): "w50i::p25_ddc50_imma_kernel<true>",
+           ("u8", 5, "w5i"): "w5i::p25_ddc5_imma_kernel<false>", ("cf32", 50, "fast"): "fast::p25_ddc_fm_stream_kernel",
+           ("u8", 50, "w50i_pw"): "w50i::p25_ddc50_imma_kernel<true>",
            ("u8", 50, "w50i"): "w50i::p25_ddc50_imma_kernel<false>"}
 
 
@@ -87,17 +88,17 @@ def _route(fmt: str, dec: int, a0: int, n: int) -> str:
     u8 = fmt == "u8"
     aligned = n % (8 if u8 else 2) == 0
     n_out = (a0 + n) // dec - a0 // dec
-    if dec == 5 and aligned and n_out > 0 and a0 >= HT[5] and n >= HT[5]:
+    if dec == 5 and aligned and n_out > 0 and a0 >= HT[5]:
         return "w5i" if u8 else "w5"
     if dec == 50 and not u8 and aligned and a0 % 2 == 0 and n_out > 0:
         return "fast"
     if dec == 50 and u8 and aligned and n_out > 0 and a0 >= HT[50]:
-        return "w50i" if n >= HT[50] else "fast"
+        return "w50i"
     return "generic"
 
 
 def _generic_segments(dec: int, n_out: int, n_streams: int, n_sm: int) -> int:
-    """p25cu_demod's segment split for the generic kernel (p25cu_api.cu)."""
+    """The generic kernel's segment split (its launcher in ddc_fm.cu)."""
     mb = 64 if dec == 50 else 256
     iters = -(-n_out // mb)
     want = max(1, min(n_sm * 16 // n_streams, iters // 8))
